@@ -24,6 +24,11 @@ A "step" is one pass of the hot path over that job.
           csrmm_cfg3 (sharded; replicated and all-gathered B), csrgemv_N/T_cfg4, csrcsc_cfg4, kmeans_cfg5 (with the
           NCCL allreduce at N > 1), each with roofline, e2e (host buffers, byte counts), cpu_baseline and a parity
           figure on the timed buffers; plus the pinned PCIe bandwidth of all ranks copying at once.
+
+--steps K sets the number of timed steps of both gemm legs.  --dump-outputs DIR writes, after the timed steps,
+what the last step of each leg returned: DIR/gemm_C_rows.npy (bof_sgemm_f32) and DIR/host_gemm_C_rows.npy
+(bof_host_gemm), fp32, the same DUMP_ROWS seeded rows of C in every run (rank 0's row block when N > 1).  The
+inputs come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,6 +54,14 @@ M_FULL = N_FULL = K_FULL = 32768
 # ncu --set full capture summarised in profiles/ (None until that capture exists)
 NCU_TRAFFIC_BYTES = 275551000000 + 4630000000  # profiles/r02/t14_per_launch_all_configs.txt (gemm3xtf32_kernel<2,0,1,1>, one launch)
 TILE = 8192  # reference GEMM_BLK_SIZE (CMakeLists.txt:46-50 of the reference)
+DUMP_ROWS = 128  # rows of C dumped per leg: 2 x 128 x 32768 fp32 = 32 MiB at the full size
+
+
+def dump_rows(m: int):
+    """The rows of an m-row C that --dump-outputs writes: a fixed seeded sample, sorted."""
+    import numpy as np
+
+    return np.sort(np.random.default_rng(0x5EED00D0).choice(m, size=min(m, DUMP_ROWS), replace=False))
 
 
 def peaks():
@@ -354,7 +367,13 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink cfg-3/4/5 (debug only; invalid as a bench value)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="leave the process on all CPUs (A/B of the NUMA binding)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write sampled rows of C from the last timed step of each gemm "
+                                                          "leg as DIR/<name>.npy (fp32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -468,6 +487,10 @@ def main():
     ii = torch.randint(0, Mr, (64,), device="cuda"); jj = torch.randint(0, Ng, (64,), device="cuda")
     ref = (A[ii].double() * B[:, jj].t().double()).sum(1)
     spot = float(((Cd[ii, jj].double() - ref).abs() / ref.abs()).max())
+    dumps = {}
+    if args.dump_outputs:
+        rows = torch.from_numpy(dump_rows(Mr))
+        dumps["gemm_C_rows"] = Cd[rows.to(Cd.device)].cpu().numpy()
     del A, B, Cd, ws
     torch.cuda.empty_cache()
 
@@ -482,7 +505,7 @@ def main():
         for r0 in range(0, host.shape[0], 4096):
             host[r0:r0 + 4096].copy_(torch.rand((min(4096, host.shape[0] - r0), host.shape[1]), device="cuda", generator=gfill))
     torch.cuda.synchronize()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     from bof_b200 import dist as bdist
     if world > 1:
         bdist.init_comm(ctx)   # the library's own communicator rank: panel broadcasts of B on its collective stream
@@ -519,6 +542,8 @@ def main():
     i0 = int(torch.randint(0, Mr, (1,))); j0 = int(torch.randint(0, Ng, (1,)))
     ref0 = float((Ah[i0].double() * Bh[:, j0].double()).sum())
     e2e["spot_rel_err"] = abs(float(Ch[i0, j0]) - ref0) / abs(ref0)
+    if args.dump_outputs:
+        dumps["host_gemm_C_rows"] = Ch[rows].numpy()
     del Ah, Bh, Ch
 
     torch.cuda.empty_cache()
@@ -538,6 +563,11 @@ def main():
         e2e["bound_note"] = ("per-GPU bytes of this run / pinned-copy rates measured in this run with all ranks copying at once "
                              "(extra.pcie): H2D alone, and H2D + D2H at the both-directions rate")
     if rank == 0:
+        if args.dump_outputs:
+            out = Path(args.dump_outputs)
+            out.mkdir(parents=True, exist_ok=True)
+            for name, arr in dumps.items():
+                np.save(out / f"{name}.npy", arr)
         line = {
             "metric": "gemm_gflops", "value": value, "unit": "GFLOP/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": t_dev * 1e3, "higher_is_better": True, "scaling": "strong",

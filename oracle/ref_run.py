@@ -31,7 +31,7 @@ def available(suffix: str = "") -> bool:
 def exe(name: str, suffix: str = "") -> str:
     p = _REF / f"{name}{suffix}"
     if not p.exists():
-        raise FileNotFoundError(f"{p} missing: run `make -C oracle -f Makefile.ref` where /root/reference exists")
+        raise FileNotFoundError(f"{p} missing: run `make -C oracle -f Makefile.ref REF=<reference sources>`")
     return str(p)
 
 

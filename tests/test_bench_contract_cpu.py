@@ -23,6 +23,12 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "GFLOP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_rejects_zero_steps():
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     """Under torchrun only rank 0 runs the CPU arm; the other ranks exit 0 without output."""
     import os

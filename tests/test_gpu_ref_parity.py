@@ -1,6 +1,6 @@
 """GPU parity against the REFERENCE ITSELF: the CUDA path, called through the C ABI host entry points, is compared
 with (i) tests/golden/golden_ref.npz -- outputs written by the reference's own binaries -- and (ii) where
-oracle/_ref travelled to this box, live runs of those binaries on fresh, larger inputs (in_mem_* = the bare MKL
+oracle/_ref has been built, live runs of those binaries on fresh, larger inputs (in_mem_* = the bare MKL
 call; flash drivers = flash::gemm / csrmm / csrgemv / csrcsc through the reference's scheduler and file handles).
 Tolerances are BASELINE.json's: relative Frobenius <= 1e-5 for gemm / csrmm / csrgemv / centroids, bit-exact for
 csrcsc and for k-means assignments on ties-free points."""
@@ -12,7 +12,8 @@ from golden_ref import G, TOL, csrcsc_cases, csrgemv_cases, csrmm_cases, gemm_ca
 from oracle import ref_run as rr
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not (rr.available() and rr.available("_small")), reason="oracle/_ref not on this box")
+needs_ref = pytest.mark.skipif(not (rr.available() and rr.available("_small")),
+                               reason="oracle/_ref not built (make -C oracle -f Makefile.ref REF=<reference sources>)")
 
 
 @pytest.mark.parametrize("case", list(gemm_cases()), ids=lambda c: c[0])

@@ -1,7 +1,7 @@
 """CPU tests that PIN THE ORACLE TO THE REFERENCE: oracle/oracle.c against tests/golden/golden_ref.npz, whose
 outputs were written by the reference's own binaries (unmodified sources built by oracle/Makefile.ref), and --
-where oracle/_ref exists (this container; it also travels to the GPU box) -- against live runs of those binaries
-on fresh inputs, including sizes that take several tiles of the default build."""
+where oracle/_ref has been built (make -C oracle -f Makefile.ref REF=<reference sources>) -- against live runs of
+those binaries on fresh inputs, including sizes that take several tiles of the default build."""
 import numpy as np
 import pytest
 
@@ -10,7 +10,7 @@ from golden_ref import G, TOL, csrcsc_cases, csrgemv_cases, csrmm_cases, gemm_ca
 from oracle import ref_run as rr
 
 needs_ref = pytest.mark.skipif(not (rr.available() and rr.available("_small")),
-                               reason="oracle/_ref not built (needs /root/reference: make -C oracle -f Makefile.ref)")
+                               reason="oracle/_ref not built (make -C oracle -f Makefile.ref REF=<reference sources>)")
 
 
 @pytest.mark.parametrize("case", list(gemm_cases()), ids=lambda c: c[0])
