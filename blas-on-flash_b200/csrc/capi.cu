@@ -238,7 +238,7 @@ int bof_kmeans_assign(bof_ctx* ctx, void* stream, int64_t npoints, int64_t ncent
   ep.argmin_out = assign;
   const int cg = ctx->cfg.gemm_force_path == 1 ? 1 : 2;
   return launch_gemm_tc(ctx, s, cg, npoints, ncenters, dim, kp, reinterpret_cast<const float*>(pp),
-                        reinterpret_cast<const float*>(pp + plane_bytes(npoints, kp)), c_hi, c_lo, ep, 0);
+                        reinterpret_cast<const float*>(pp + plane_bytes(npoints, kp)), c_hi, c_lo, ep, k_chunk_of(ctx));
 }
 
 size_t bof_kmeans_reduce_workspace_bytes(int64_t npoints, int64_t ncenters, int64_t dim) {

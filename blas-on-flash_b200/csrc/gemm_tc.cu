@@ -645,12 +645,34 @@ __device__ __forceinline__ float rna_tf32(float x) {
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
   return __uint_as_float(u);
 }
-__device__ __forceinline__ void split1(float x, float& hi, float& lo) {
-  hi = rna_tf32(x);
-  lo = rna_tf32(x - hi);
-}
-__device__ __forceinline__ uint16_t bf16_bits(float x) {
-  return __bfloat16_as_ushort(__float2bfloat16_rn(x));
+
+// The planes of one operand element, for both splits: hi (tf32), lo = rna_tf32(x - hi) (the gemm_split = 1 plane)
+// and the hybrid pair bh = bf16(hi), bl = bf16(x - hi).  Both split kernels call this one function.
+//   - Non-finite x: hi = x and every residual 0, so that the cross terms vanish and hi*hi carries the IEEE Inf / NaN
+//     (x - hi would be NaN).
+//   - |x| >= 0x1.ffep127 (bits 0x7f7ff000): rna_tf32 would round to Inf, so hi truncates instead; x - hi stays exact
+//     and lo keeps ~2^-21 relative.
+//   - |hi| >= 0x1.ffp127 (bits 0x7f7f8000): bf16 round-to-nearest would overflow, so bh rounds toward zero (error
+//     2^-8 of a cross term that is itself ~2^-11 of the product).
+// Below these thresholds the planes are exactly rna_tf32 / bf16 round-to-nearest.
+struct SplitElem {
+  float hi, lo;
+  uint16_t bh, bl;
+};
+__device__ __forceinline__ SplitElem split_elem(float x) {
+  SplitElem s;
+  const uint32_t ax = __float_as_uint(x) & 0x7fffffffu;
+  if (ax >= 0x7f800000u) {
+    s.hi = x; s.lo = 0.f; s.bh = 0; s.bl = 0;
+    return s;
+  }
+  s.hi = ax >= 0x7f7ff000u ? __uint_as_float(__float_as_uint(x) & ~0x1fffu) : rna_tf32(x);
+  const float e = x - s.hi;  // exact in fp32
+  s.lo = rna_tf32(e);
+  const uint32_t ah = __float_as_uint(s.hi) & 0x7fffffffu;
+  s.bh = ah >= 0x7f7f8000u ? (uint16_t)(__float_as_uint(s.hi) >> 16) : __bfloat16_as_ushort(__float2bfloat16_rn(s.hi));
+  s.bl = __bfloat16_as_ushort(__float2bfloat16_rn(e));
+  return s;
 }
 // Hybrid second plane: per 32-element k group (128 bytes) 32 x bf16(hi) then 32 x bf16(lo), lo = x - hi exact.
 __device__ __forceinline__ uint8_t* combo_ptr(float* plane, int64_t r, int64_t kp, int64_t kk, bool lo_half) {
@@ -676,21 +698,16 @@ split_planes_kmajor_kernel(int64_t R, int64_t K, const float* __restrict__ src, 
       for (int u = 0; u < 4; ++u)
         if (k0 + u < K) x[u] = p[u];
     }
-    float4 h, l;
-    split1(x[0], h.x, l.x);
-    split1(x[1], h.y, l.y);
-    split1(x[2], h.z, l.z);
-    split1(x[3], h.w, l.w);
-    *reinterpret_cast<float4*>(hi + r * kp + k0) = h;
+    const SplitElem s0 = split_elem(x[0]), s1 = split_elem(x[1]), s2 = split_elem(x[2]), s3 = split_elem(x[3]);
+    *reinterpret_cast<float4*>(hi + r * kp + k0) = make_float4(s0.hi, s1.hi, s2.hi, s3.hi);
     if (!combo) {
-      *reinterpret_cast<float4*>(lo + r * kp + k0) = l;
+      *reinterpret_cast<float4*>(lo + r * kp + k0) = make_float4(s0.lo, s1.lo, s2.lo, s3.lo);
     } else {
-      const float e[4] = {x[0] - h.x, x[1] - h.y, x[2] - h.z, x[3] - h.w};  // exact in fp32
       uint2 ph, pl;
-      ph.x = bf16_bits(h.x) | ((uint32_t)bf16_bits(h.y) << 16);
-      ph.y = bf16_bits(h.z) | ((uint32_t)bf16_bits(h.w) << 16);
-      pl.x = bf16_bits(e[0]) | ((uint32_t)bf16_bits(e[1]) << 16);
-      pl.y = bf16_bits(e[2]) | ((uint32_t)bf16_bits(e[3]) << 16);
+      ph.x = s0.bh | ((uint32_t)s1.bh << 16);
+      ph.y = s2.bh | ((uint32_t)s3.bh << 16);
+      pl.x = s0.bl | ((uint32_t)s1.bl << 16);
+      pl.y = s2.bl | ((uint32_t)s3.bl << 16);
       *reinterpret_cast<uint2*>(combo_ptr(lo, r, kp, k0, false)) = ph;
       *reinterpret_cast<uint2*>(combo_ptr(lo, r, kp, k0, true)) = pl;
     }
@@ -715,15 +732,13 @@ split_planes_transpose_kernel(int64_t R, int64_t K, const float* __restrict__ sr
   for (int i = ty; i < 32; i += 8) {
     const int64_t r = r0 + i, kk = k0 + tx;
     if (r < R && kk < kp) {
-      float h, l;
-      const float x = tile[tx][i];
-      split1(x, h, l);
-      hi[r * kp + kk] = h;
+      const SplitElem sp = split_elem(tile[tx][i]);
+      hi[r * kp + kk] = sp.hi;
       if (!combo) {
-        lo[r * kp + kk] = l;
+        lo[r * kp + kk] = sp.lo;
       } else {
-        *reinterpret_cast<uint16_t*>(combo_ptr(lo, r, kp, kk, false)) = bf16_bits(h);
-        *reinterpret_cast<uint16_t*>(combo_ptr(lo, r, kp, kk, true)) = bf16_bits(x - h);
+        *reinterpret_cast<uint16_t*>(combo_ptr(lo, r, kp, kk, false)) = sp.bh;
+        *reinterpret_cast<uint16_t*>(combo_ptr(lo, r, kp, kk, true)) = sp.bl;
       }
     }
   }

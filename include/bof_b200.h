@@ -70,7 +70,9 @@ typedef struct bof_config {
   int32_t gemm_split;        /* operand split of the fp32 GEMM: 0 = default, 1 = 3xTF32 (lo*hi + hi*lo +
                                 hi*hi, all kind::tf32), 2 = hybrid (hi*hi kind::tf32, the two cross
                                 terms on bf16 copies, kind::f16: 2/3 of the tensor time, cross-term
-                                error <= 2^-19 relative)                                          */
+                                error <= 2^-19 relative).  With 1, an infinite input may give NaN
+                                instead of +-Inf in its own row and column of C (hi*lo = Inf * 0 where
+                                the partner is tf32-exact); other elements are unaffected.        */
   int32_t radix_max_bits;    /* digit width of the csrcsc / k-means radix passes: 0 = default 8; smaller values
                                 force more passes (test knob)                                            */
   int32_t spmv_t_atomic;     /* csrgemv 'T': 0 = default, deterministic (products sorted by column, fixed-order sums,
@@ -144,6 +146,9 @@ BOF_API int bof_idx_widen(bof_ctx* ctx, void* stream, const int32_t* in, int64_t
  * Replaces cblas_sgemm in GemmTask::execute (include/tasks/gemm_task.h:67-93); argument meaning
  * as flash::gemm (include/flash_blas.h:14-18): ord 'R'/'C', ta/tb 'N'/'T', ld* = 0 => tight
  * (src/blas/gemm.cpp:63-67).  beta == 0 => C is not read (gemm_task.h:49-53).
+ * Special values follow IEEE as cblas_sgemm does: an Inf or NaN in A, B or (beta != 0) C gives the Inf / NaN of
+ * the exact dot product in the elements it meets and leaves every other element unchanged (gemm_split = 1: see
+ * bof_config.gemm_split).  Finite inputs up to FLT_MAX keep the fp32 accuracy as long as the products are finite.
  * Needs workspace of bof_sgemm_workspace_bytes(m, n, k) bytes (the TF32 hi/lo operand planes). */
 BOF_API int bof_sgemm_f32(bof_ctx* ctx, void* stream, char ord, char ta, char tb, int64_t m, int64_t n,
                   int64_t k, float alpha, const float* A, int64_t lda, const float* B,
@@ -176,6 +181,8 @@ BOF_API int bof_row_sqnorm_f32(bof_ctx* ctx, void* stream, int64_t rows, int64_t
  * Replaces KMeansTask::execute (include/tasks/kmeans_task.h:53-82: sgemm alpha=-2 + two rank-1
  * updates) fused with the cblas_isamin scan of drivers/in_mem_kmeans.cpp:82-85 -- the P x K
  * distance matrix is never materialised.  points P x dim, centers K x dim, row-major, tight.
+ * The dot products are computed like bof_sgemm_f32's, with the same special-value contract and the same
+ * bof_config.gemm_k_chunk fold of the accumulation (dim <= 256 is one chunk at the default).
  * Needs workspace bof_kmeans_workspace_bytes(). `points_planes` is optional: a caller iterating
  * on the same points passes the buffer filled by bof_kmeans_prepare_points() to skip the
  * per-call TF32 split of the points. */
