@@ -190,6 +190,11 @@ struct GemmEpilogue {
   const float* row_add = nullptr;
   const float* col_add = nullptr;
   int32_t* argmin_out = nullptr;
+  // k-panels of one long k (plain GEMM only): each element's fold starts from carry[i * ld_carry + j] instead of 0,
+  // and raw_out stores the fold itself to C (alpha and beta are applied by the last panel only)
+  const float* carry = nullptr;
+  int64_t ld_carry = 0;
+  bool raw_out = false;
 };
 
 // Tensor-core core: acc[i, j] = sum_k P[i, k] * Q[j, k] with P = (p_hi, p_lo) M x kp planes and

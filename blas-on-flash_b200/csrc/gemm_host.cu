@@ -54,6 +54,38 @@ int64_t k_chunk_of(const bof_ctx* ctx) {
   return ctx->cfg.gemm_k_chunk == 0 ? 256 : ctx->cfg.gemm_k_chunk;
 }
 
+// rows of the canonical P operand per block of the host pipeline
+static int64_t host_row_block(const bof_ctx* ctx, int64_t Mo) {
+  int64_t rb = (int64_t)ctx->cfg.gemm_row_block;
+  rb = std::max<int64_t>(256, round_up<int64_t>(rb, 256));
+  return std::min(rb, round_up<int64_t>(Mo, 256));
+}
+
+// Device memory a host GEMM may plan with: BOF_GEMM_HBM_BUDGET=<bytes> when set (read on every call, so a test can
+// force the out-of-core plan at a small size), otherwise the free memory plus what the context already holds in
+// `slots` (slot_reserve frees a slot before it grows it).  *forced tells which.
+static size_t gemm_hbm_available(const bof_ctx* ctx, const std::vector<int>& slots, bool* forced) {
+  const char* e = getenv("BOF_GEMM_HBM_BUDGET");
+  *forced = e != nullptr && *e != '\0';
+  if (*forced) return (size_t)strtoull(e, nullptr, 10);
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); return SIZE_MAX; }  // unknown: plan resident
+  for (int sl : slots) free_b += ctx->slot_bytes[sl];
+  return free_b;
+}
+
+// The slots of the resident host GEMM plan and the bytes it reserves in each (kGemmRing P generations at most).
+static std::vector<std::pair<int, size_t>> resident_gemm_slots(const bof_ctx* ctx, const Canon& cn, bool with_terms) {
+  const int64_t K = std::max<int64_t>(cn.K, 1), kp = padded_k(cn.K), rb = host_row_block(ctx, cn.Mo);
+  const int ngen = (int)std::min<int64_t>(kGemmRing, ceil_div<int64_t>(cn.Mo, rb));
+  std::vector<std::pair<int, size_t>> v = {
+      {S_DENSE, (size_t)cn.No * K * 4}, {S_DENSE_T, 2 * plane_bytes(cn.No, kp)},
+      {S_PPLANES, 2 * (size_t)ngen * plane_bytes(rb, kp)}, {S_GCBLK, (size_t)ngen * rb * cn.No * 4}};
+  for (int g = 0; g < ngen; ++g) v.push_back({S_PRAW + g, (size_t)rb * K * 4});
+  if (with_terms) v.push_back({S_MISC, (size_t)(cn.Mo + cn.No) * 4});
+  return v;
+}
+
 // GEMM on device-resident canonical operands with a caller-provided plane workspace.
 int gemm_canon_device(bof_ctx* ctx, cudaStream_t s, const Canon& c, float alpha, float beta, float* C,
                       void* ws, size_t ws_bytes) {
@@ -83,6 +115,180 @@ int gemm_canon_device(bof_ctx* ctx, cudaStream_t s, const Canon& c, float alpha,
 }  // namespace bof
 
 using namespace bof;
+
+// Out-of-core plan of bof_host_gemm / bof_host_kmeans_dist, for operands whose resident plan does not fit the device.
+// C is computed in super-blocks of S rows whose fp32 fold stays on the device for the whole k extent.  k is walked
+// in panels of L elements, L a multiple of the fold chunk (launch_gemm_tc folds TMEM into fp32 every chunk), and each
+// panel's launch resumes the fold the previous panel stored: the additions are the resident plan's, in its order,
+// so the result is the same bits whatever the budget.  Per (super-block, panel) Q's panel is uploaded and split once
+// into one of two buffers, so that panel p + 1 uploads while panel p multiplies; P's row blocks stream through the
+// ring of kGemmRing generations, which cycles over (panel, row block) items.  The last panel applies alpha, beta
+// (C0 read from its own buffer) and the k-means terms, and the rows of C are downloaded behind it.
+// PCIe: H2D = sz(P) + n_super * sz(Q) [+ sz(C) when beta != 0], D2H = sz(C).
+static int host_gemm_ooc(bof_ctx* ctx, const Canon& cn, int cg, float alpha, float beta, float* c, const float* term_rows,
+                         const float* term_cols, int row_first, bool forced) {
+  constexpr int NB = kGemmRing;
+  const int64_t Mo = cn.Mo, No = cn.No, K = cn.K;
+  const int64_t kc = k_chunk_of(ctx);
+  const int64_t unit = 32 * (kc <= 0 ? 1 : std::max<int64_t>(1, kc / 32));  // a panel starts on a fold-chunk boundary
+  const bool with_terms = term_rows != nullptr;
+  const int64_t rb0 = host_row_block(ctx, Mo);
+  const size_t c_row = (size_t)No * 4 * (beta != 0.f ? 2 : 1);   // fold [+ C0] per row of a super-block
+  const size_t terms = with_terms ? (size_t)(Mo + No) * 4 : 0;
+  auto footprint = [&](int64_t S, int64_t rb, int64_t L) -> size_t {
+    return (size_t)S * c_row + terms + 2 * ((size_t)No * L * 4 + 2 * plane_bytes(No, L)) +
+           (size_t)NB * ((size_t)rb * L * 4 + 2 * plane_bytes(rb, L));
+  };
+  // the slots this plan uses; what they hold counts as available, and what it does not need of them is released
+  const std::vector<int> ids = {S_DENSE, S_DENSE_T, S_PRAW, S_PRAW + 1, S_PRAW + 2, S_PRAW + 3, S_PRAW + 4,
+                                S_PPLANES, S_GCBLK, S_CBLK, S_MISC};
+  static_assert(NB == 5, "the slot list holds kGemmRing P generations");
+  bool unused;
+  size_t avail = gemm_hbm_available(ctx, ids, &unused);
+  if (!forced) avail -= std::min<size_t>(avail / 4, (size_t)1 << 30);  // allocation granularity, kernel workspaces
+
+  const int64_t s_units = ceil_div<int64_t>(Mo, 256);
+  const size_t need_min = footprint(std::min<int64_t>(Mo, 256), 256, unit);
+  if (need_min > avail)
+    return fail(ctx, BOF_ENOMEM,
+                "gemm: the operands exceed device memory and the out-of-core plan needs at least %zu bytes "
+                "(256 rows of C, k-panels of %lld), %zu available", need_min, (long long)unit, avail);
+  // S first, as large as fits with the shortest panel: every extra super-block re-streams Q
+  int64_t lo = 1, hi = s_units;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) / 2;
+    if (footprint(std::min(Mo, mid * 256), std::min(rb0, mid * 256), unit) <= avail) lo = mid; else hi = mid - 1;
+  }
+  // whole row blocks of at most rb0 rows per super-block
+  const int64_t blocks = ceil_div<int64_t>(lo * 256, rb0);
+  const int64_t rb = lo / blocks * 256;
+  const int64_t S = std::min(Mo, rb * blocks);
+  // then L as long as the rest allows, evened out over the panels
+  lo = 1; hi = ceil_div<int64_t>(K, unit);
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) / 2;
+    if (footprint(S, rb, mid * unit) <= avail) lo = mid; else hi = mid - 1;
+  }
+  const int64_t npan = ceil_div<int64_t>(K, lo * unit);
+  const int64_t L = round_up<int64_t>(ceil_div<int64_t>(K, npan), unit);
+
+  // ---- buffers ----
+  const size_t qpb = plane_bytes(No, L), ppb = plane_bytes(rb, L);
+  std::vector<std::pair<int, size_t>> need = {{S_DENSE, (size_t)No * L * 8}, {S_DENSE_T, 4 * qpb},
+                                              {S_PPLANES, 2 * (size_t)NB * ppb}, {S_GCBLK, (size_t)S * No * 4},
+                                              {S_CBLK, beta != 0.f ? (size_t)S * No * 4 : 0}, {S_MISC, terms}};
+  for (int g = 0; g < NB; ++g) need.push_back({S_PRAW + g, (size_t)rb * L * 4});
+  bool synced = false;
+  for (auto& sb : need) {
+    if (ctx->slot_bytes[sb.first] <= sb.second) continue;
+    if (!synced) { BOF_CUDA(ctx, cudaDeviceSynchronize()); synced = true; }   // a slot may still be in use by queued work
+    BOF_CUDA(ctx, cudaFree(ctx->slot_ptr[sb.first]));
+    ctx->slot_ptr[sb.first] = nullptr;
+    ctx->slot_bytes[sb.first] = 0;
+  }
+  float* qraw; float* praw[NB]; float* fold; float* c0 = nullptr; float* term_d = nullptr;
+  void* qpl; void* ppl;
+  BOF_TRY(slot_reserve(ctx, S_DENSE, (size_t)No * L * 2, &qraw));
+  BOF_TRY(slot_reserve(ctx, S_DENSE_T, 4 * qpb, &qpl));
+  BOF_TRY(slot_reserve(ctx, S_PPLANES, 2 * (size_t)NB * ppb, &ppl));
+  for (int g = 0; g < NB; ++g) BOF_TRY(slot_reserve(ctx, S_PRAW + g, (size_t)rb * L, &praw[g]));
+  BOF_TRY(slot_reserve(ctx, S_GCBLK, (size_t)S * No, &fold));
+  if (beta != 0.f) BOF_TRY(slot_reserve(ctx, S_CBLK, (size_t)S * No, &c0));
+  auto plane = [](void* base, size_t bytes, int64_t i) { return reinterpret_cast<float*>(static_cast<uint8_t*>(base) + i * bytes); };
+  auto q_hi = [&](int b) { return plane(qpl, qpb, 2 * b); };
+  auto q_lo = [&](int b) { return plane(qpl, qpb, 2 * b + 1); };
+  auto p_hi = [&](int g) { return plane(ppl, ppb, g); };
+  auto p_lo = [&](int g) { return plane(ppl, ppb, NB + g); };
+
+  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice;
+  if (with_terms) {
+    BOF_TRY(slot_reserve(ctx, S_MISC, (size_t)(Mo + No), &term_d));
+    BOF_TRY(copy1d(ctx, term_d, term_rows, (size_t)Mo * 4, H2D, ctx->h2d));
+    BOF_TRY(copy1d(ctx, term_d + Mo, term_cols, (size_t)No * 4, H2D, ctx->h2d));
+    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, 3), ctx->h2d));
+    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, 3), 0));
+  }
+  // rows [r0, r1) x k [k0, k1) of a canonical operand as a tight device block; returns its strides
+  auto upload = [&](const float* src, int64_t s_r, int64_t s_k, int64_t r0, int64_t r1, int64_t k0, int64_t k1, float* dst,
+                    int64_t* d_sr, int64_t* d_sk) -> int {
+    const int64_t rows = r1 - r0, len = k1 - k0;
+    if (s_k == 1) {
+      *d_sr = len; *d_sk = 1;
+      return copy2d(ctx, dst, (size_t)len * 4, src + r0 * s_r + k0, (size_t)s_r * 4, (size_t)len * 4, (size_t)rows, H2D, ctx->h2d);
+    }
+    *d_sr = 1; *d_sk = rows;  // stored k-major: rows [k0, k1) of a [K x ld] matrix, columns [r0, r1)
+    return copy2d(ctx, dst, (size_t)rows * 4, src + r0 + k0 * s_k, (size_t)s_k * 4, (size_t)rows * 4, (size_t)len, H2D, ctx->h2d);
+  };
+
+  // events: 8+g P item uploaded, 16+g P item split, 24+g rows of C final, 32+g rows of C downloaded, 40+b Q panel
+  // uploaded, 42+b Q buffer released, 44 C0 rows uploaded
+  constexpr int EV_UP = 8, EV_SPLIT = 16, EV_DONE = 24, EV_DOWN = 32, EV_QUP = 40, EV_QFREE = 42, EV_C0 = 44;
+  bool p_used[NB] = {}, q_used[2] = {}, down_used[NB] = {};
+  uint64_t down_ticket[NB] = {};
+  int64_t item = 0, qseq = 0;
+  for (int64_t s0 = 0; s0 < Mo; s0 += S) {
+    const int64_t s1 = std::min(Mo, s0 + S);
+    const int64_t nb = ceil_div<int64_t>(s1 - s0, rb);
+    // the rows of C of the previous super-block leave the buffer this one writes its result into first
+    for (int g = 0; g < NB; ++g) {
+      if (!down_used[g]) continue;
+      d2h_fence(ctx, down_ticket[g]);
+      BOF_CUDA(ctx, cudaStreamWaitEvent(beta != 0.f ? ctx->h2d : ctx->compute, get_event(ctx, EV_DOWN + g), 0));
+    }
+    if (beta != 0.f) {
+      BOF_TRY(copy2d(ctx, c0, (size_t)No * 4, c + s0 * cn.ldc, (size_t)cn.ldc * 4, (size_t)No * 4, (size_t)(s1 - s0), H2D, ctx->h2d));
+      BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_C0), ctx->h2d));
+    }
+    for (int64_t p = 0; p < npan; ++p, ++qseq) {
+      const int64_t k0 = p * L, k1 = std::min(K, k0 + L), len = k1 - k0, kpp = padded_k(len);
+      const bool first = p == 0, last = p == npan - 1;
+      const int b = (int)(qseq & 1);
+      float* qbuf = qraw + (size_t)b * No * L;
+      if (q_used[b]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, EV_QFREE + b), 0));
+      int64_t q_sr, q_sk;
+      BOF_TRY(upload(cn.qsrc, cn.q_sr, cn.q_sk, 0, No, k0, k1, qbuf, &q_sr, &q_sk));
+      BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_QUP + b), ctx->h2d));
+      trace_mark(ctx, ctx->h2d, "h2d: Q k-panel landed", (int)p);
+      for (int64_t i = 0; i < nb; ++i, ++item) {
+        const int g = (int)(item % NB);
+        const int64_t r0 = s0 + i * rb, rows = std::min(s1, r0 + rb) - r0;
+        if (p_used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, EV_SPLIT + g), 0));  // raw P consumed
+        int64_t p_sr, p_sk;
+        BOF_TRY(upload(cn.psrc, cn.p_sr, cn.p_sk, r0, r0 + rows, k0, k1, praw[g], &p_sr, &p_sk));
+        BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_UP + g), ctx->h2d));
+        if (i == 0) {
+          BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_QUP + b), 0));
+          BOF_TRY(launch_split_planes(ctx, ctx->compute, No, len, qbuf, q_sr, q_sk, q_hi(b), q_lo(b), kpp));
+        }
+        BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_UP + g), 0));
+        BOF_TRY(launch_split_planes(ctx, ctx->compute, rows, len, praw[g], p_sr, p_sk, p_hi(g), p_lo(g), kpp));
+        BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_SPLIT + g), ctx->compute));
+        p_used[g] = true;
+        float* fold_rows = fold + (size_t)(r0 - s0) * No;
+        float* out = (last && beta != 0.f) ? c0 + (size_t)(r0 - s0) * No : fold_rows;
+        if (last && beta != 0.f && i == 0) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_C0), 0));
+        GemmEpilogue ep;
+        ep.alpha = alpha; ep.beta = beta; ep.C = out; ep.ldc = No;
+        ep.carry = first ? nullptr : fold_rows; ep.ld_carry = No;
+        ep.raw_out = !last;
+        BOF_TRY(launch_gemm_tc(ctx, ctx->compute, cg, rows, No, len, kpp, p_hi(g), p_lo(g), q_hi(b), q_lo(b), ep, kc));
+        if (!last) continue;
+        if (with_terms)
+          BOF_TRY(launch_add_outer_terms(ctx, ctx->compute, out, rows, No, No, term_d + r0, term_d + Mo, row_first));
+        if (down_used[g]) d2h_fence(ctx, down_ticket[g]);  // EV_DONE + g is waited on by that download
+        BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_DONE + g), ctx->compute));
+        BOF_TRY(d2h_transfer(ctx, c + r0 * cn.ldc, (size_t)cn.ldc * 4, out, (size_t)No * 4, (size_t)No * 4, (size_t)rows,
+                             ctx->d2h, get_event(ctx, EV_DONE + g), get_event(ctx, EV_DOWN + g), &down_ticket[g]));
+        down_used[g] = true;
+      }
+      BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_QFREE + b), ctx->compute));
+      q_used[b] = true;
+    }
+  }
+  BOF_TRY(sync_all(ctx));
+  trace_dump(ctx, "bof_host_gemm (out of core)");
+  return BOF_OK;
+}
 
 extern "C" {
 
@@ -125,6 +331,25 @@ static int host_gemm_impl(bof_ctx* ctx, char ord, char ta, char tb, int64_t m, i
     return copy2d(ctx, dst, (size_t)rows * 4, src + r0, (size_t)s_k * 4, (size_t)rows * 4, (size_t)K, H2D, s);
   };
 
+  const bool with_terms = term_m != nullptr && term_n != nullptr;
+  const bool canon_rows_are_m = ord == 'R';
+  if (tensor && !q_on_device && !dist_call) {
+    // Operands whose resident plan does not fit the device take the out-of-core plan; every call that fits stays here.
+    std::vector<std::pair<int, size_t>> need = resident_gemm_slots(ctx, cn, with_terms);
+    std::vector<int> ids;
+    size_t total = 0;
+    for (auto& sb : need) { ids.push_back(sb.first); total += sb.second; }
+    bool forced;
+    const size_t avail = gemm_hbm_available(ctx, ids, &forced);
+    if (total > avail) {
+      const float* term_rows = with_terms ? (canon_rows_are_m ? term_m : term_n) : nullptr;
+      const float* term_cols = with_terms ? (canon_rows_are_m ? term_n : term_m) : nullptr;
+      BOF_TRY(host_gemm_ooc(ctx, cn, cg, alpha, beta, c, term_rows, term_cols, canon_rows_are_m ? 1 : 0, forced));
+      stats_end(ctx);
+      return call_guard.done();
+    }
+  }
+
   // ---- buffers ----
   float* qraw = nullptr;
   float* q_hi = nullptr;
@@ -165,9 +390,7 @@ static int host_gemm_impl(bof_ctx* ctx, char ord, char ta, char tb, int64_t m, i
     q_hi = static_cast<float*>(p);
     q_lo = reinterpret_cast<float*>(static_cast<uint8_t*>(p) + qb);
   }
-  int64_t rb = (int64_t)ctx->cfg.gemm_row_block;
-  rb = std::max<int64_t>(256, round_up<int64_t>(rb, 256));
-  rb = std::min(rb, round_up<int64_t>(cn.Mo, 256));
+  int64_t rb = host_row_block(ctx, cn.Mo);
   // a rank's shard of a multi-GPU job can be a single block: cut it into four so that the first MMAs start after a
   // quarter of it has landed and the C slabs leave earlier
   if (dist_q && comm_world(ctx) > 1 && cn.Mo <= 4 * rb) rb = std::max<int64_t>(1024, round_up<int64_t>(ceil_div<int64_t>(cn.Mo, 4), 256));
@@ -196,8 +419,6 @@ static int host_gemm_impl(bof_ctx* ctx, char ord, char ta, char tb, int64_t m, i
   // device before it is downloaded.  In canonical (row-major output) form the rows are m for 'R', n for 'C'.
   float* term_rows_d = nullptr;
   float* term_cols_d = nullptr;
-  const bool with_terms = term_m != nullptr && term_n != nullptr;
-  const bool canon_rows_are_m = ord == 'R';
   if (with_terms) {
     float* t;
     BOF_TRY(slot_reserve(ctx, S_MISC, (size_t)(cn.Mo + cn.No), &t));

@@ -69,6 +69,12 @@ struct Params {
   // operand panels stay inside L2 (measured without it at 32768^3: L2 hit rate 36%, DRAM 59% busy).
   uint32_t* sync_counters;
   int32_t sync_kb;
+  // FOLD variant (EPI_GEMM, k-panels of an out-of-core GEMM): chunk 0 of every element starts from
+  // carry[row * ld_carry + col] when carry != nullptr; raw_out != 0 stores the un-scaled fold to C
+  // (no alpha, no beta, C not read), so that the next k-panel can resume it.
+  const float* carry;
+  int64_t ld_carry;
+  int32_t raw_out;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -281,7 +287,7 @@ constexpr size_t SMEM_BYTES = (size_t)STAGES * STAGE_BYTES + sizeof(SmemTail) + 
 // ---------------------------------------------------------------------------------------------
 // The kernel
 // ---------------------------------------------------------------------------------------------
-template <int CG, int EPI, bool CHUNKED, bool HYB>
+template <int CG, int EPI, bool CHUNKED, bool HYB, bool FOLD = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm3xtf32_kernel(const __grid_constant__ CUtensorMap map_p_hi, const __grid_constant__ CUtensorMap map_p_lo,
                   const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ CUtensorMap map_q_lo,
@@ -292,6 +298,7 @@ gemm3xtf32_kernel(const __grid_constant__ CUtensorMap map_p_hi, const __grid_con
   constexpr uint32_t TMEM_COLS = 2 * BLOCK_N;
   constexpr uint32_t IDESC = make_idesc(BLOCK_M * CG, BLOCK_N, 2u);
   constexpr uint32_t IDESC_BF16 = make_idesc(BLOCK_M * CG, BLOCK_N, 1u);
+  static_assert(!FOLD || (EPI == EPI_GEMM && CHUNKED), "the fold carry exists for the chunked GEMM epilogue only");
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -475,7 +482,13 @@ gemm3xtf32_kernel(const __grid_constant__ CUtensorMap map_p_hi, const __grid_con
             tmem_ld32(taddr + g * 32, v);
             tmem_ld_wait();
             if constexpr (CHUNKED) {
-              if (c == 0) {
+              if (FOLD && c == 0 && prm.carry != nullptr && row < prm.M) {
+                // resume the fold of the previous k-panel: same additions, in the same order, as one long k
+                const float* krow = prm.carry + row * prm.ld_carry + col0 + g * 32;
+#pragma unroll
+                for (int j = 0; j < 32; ++j)
+                  acc[g * 32 + j] = (col0 + g * 32 + j < prm.N) ? krow[j] + __uint_as_float(v[j]) : __uint_as_float(v[j]);
+              } else if (c == 0) {
 #pragma unroll
                 for (int j = 0; j < 32; ++j) acc[g * 32 + j] = __uint_as_float(v[j]);
               } else {
@@ -521,7 +534,9 @@ gemm3xtf32_kernel(const __grid_constant__ CUtensorMap map_p_hi, const __grid_con
               float* crow = prm.C + row * prm.ldc + col0;
 #pragma unroll
               for (int j = 0; j < EPI_COLS; ++j) {
-                if (col0 + j < prm.N) {
+                if (FOLD && prm.raw_out) {
+                  if (col0 + j < prm.N) crow[j] = acc[j];
+                } else if (col0 + j < prm.N) {
                   float r = prm.alpha * acc[j];
                   if (prm.beta != 0.f) r = fmaf(prm.beta, crow[j], r);
                   crow[j] = r;
@@ -820,9 +835,9 @@ int make_plane_map(bof_ctx* ctx, CUtensorMap* map, const float* plane, int64_t r
   return BOF_OK;
 }
 
-template <int CG, int EPI, bool CHUNKED, bool HYB>
+template <int CG, int EPI, bool CHUNKED, bool HYB, bool FOLD = false>
 int launch_variant(bof_ctx* ctx, cudaStream_t s, const CUtensorMap* maps, const tc::Params& prm, int num_items) {
-  auto kern = tc::gemm3xtf32_kernel<CG, EPI, CHUNKED, HYB>;
+  auto kern = tc::gemm3xtf32_kernel<CG, EPI, CHUNKED, HYB, FOLD>;
   static PerDeviceOnce attr_set;
   if (attr_set.need(ctx->device)) {
     BOF_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
@@ -912,8 +927,13 @@ int launch_gemm_tc(bof_ctx* ctx, cudaStream_t s, int cta_group, int64_t M, int64
   prm.row_add = ep.row_add;
   prm.col_add = ep.col_add;
   prm.argmin_out = ep.argmin_out;
+  prm.carry = ep.carry;
+  prm.ld_carry = ep.ld_carry;
+  prm.raw_out = ep.raw_out ? 1 : 0;
+  const bool fold = ep.carry != nullptr || ep.raw_out;
   if (argmin)
     BOF_REQUIRE(ctx, ep.row_add && ep.col_add && ep.argmin_out, "gemm_tc: argmin epilogue needs norms and an output");
+  BOF_REQUIRE(ctx, !(argmin && fold), "gemm_tc: the fold carry needs the GEMM epilogue");
   const bool chunked = prm.kb_per_chunk < prm.num_kb;
   const int num_items = argmin ? prm.tiles_m : prm.tiles_m * prm.tiles_n;
   // wave lock-step only pays when a tile's k-panel outgrows L2 and there is more than one wave
@@ -941,6 +961,14 @@ int launch_gemm_tc(bof_ctx* ctx, cudaStream_t s, int cta_group, int64_t M, int64
   }
 
   const bool hyb = hybrid_split(ctx);
+  if (fold) {  // a k-panel shorter than one chunk still goes through the chunked epilogue that holds the fold
+    if (cta_group == 2) {
+      if (hyb) return launch_variant<2, tc::EPI_GEMM, true, true, true>(ctx, s, maps, prm, num_items);
+      return launch_variant<2, tc::EPI_GEMM, true, false, true>(ctx, s, maps, prm, num_items);
+    }
+    if (hyb) return launch_variant<1, tc::EPI_GEMM, true, true, true>(ctx, s, maps, prm, num_items);
+    return launch_variant<1, tc::EPI_GEMM, true, false, true>(ctx, s, maps, prm, num_items);
+  }
 #define BOF_TC(CG, EPI, CH)                                                            \
   do {                                                                                 \
     if (hyb) return launch_variant<CG, EPI, CH, true>(ctx, s, maps, prm, num_items);   \
