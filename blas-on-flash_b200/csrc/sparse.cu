@@ -37,12 +37,13 @@ __device__ __forceinline__ void fma4(float4& acc, float v, const float4& b) {
 //     warp order, or
 //   * every warp of the grid (rows beyond max(16384, 64 x the mean row length)), block partials combined through a
 //     fixed workspace in block order after a grid barrier (all blocks are co-resident),
-// so the result is deterministic and no row occupies one warp for more than kMidRow nonzeros.  No host round trip,
-// no size-dependent workspace; a matrix without such rows pays one memset and one empty launch.
+// so no row occupies one warp for more than kMidRow nonzeros.  The result is deterministic: which tree sums a row
+// depends only on its length and the launch's mean, never on the order in which rows were filed (each list has room
+// for every row of the launch, so nothing spills from one path to the other).  No host round trip; the workspace is
+// two m-entry lists and a grid of partials; a matrix without such rows pays one memset and one empty launch.
 constexpr int kMidRow = 1024;            // nonzeros above which a row leaves the row-group kernel
 constexpr int kLongRowMin = 16384;       // rows above max(this, kLongRowFactor x mean) are spread over the whole grid
 constexpr int kLongRowFactor = 64;
-constexpr int kLongCap = 4096;           // rows the grid-wide path takes per launch (more spill into the block path)
 
 struct LongRows {
   uint32_t* counters;   // [0] rows in mid_list, [1] rows in long_list, [2..3] grid barrier, [4] work ticket
@@ -78,16 +79,14 @@ spmm_csr_rm_vec_kernel(int64_t m, int64_t k, float alpha, const float* __restric
     end = offs[row + 1] - base;
   }
   if (lr.counters != nullptr && end - beg > kMidRow) {
-    // deferred to spmm_long_rows_kernel: every column chunk skips the row, chunk 0 files it.  The lists cannot
-    // overflow (mid_list has m entries; a full long_list spills into mid_list, whose path handles any length).
+    // deferred to spmm_long_rows_kernel: every column chunk skips the row, chunk 0 files it.  Neither list can
+    // overflow: each has room for all m rows.
     if (sl == 0 && blockIdx.y == 0) {
       const int64_t mean = (offs[m] - base) / m;
-      bool is_long = end - beg > max((int64_t)kLongRowMin, (int64_t)kLongRowFactor * mean);
-      if (is_long) {
-        const uint32_t got = atomicAdd(&lr.counters[1], 1u);
-        if (got < (uint32_t)kLongCap) lr.long_list[got] = (int32_t)row; else is_long = false;
-      }
-      if (!is_long) lr.mid_list[atomicAdd(&lr.counters[0], 1u)] = (int32_t)row;
+      if (end - beg > max((int64_t)kLongRowMin, (int64_t)kLongRowFactor * mean))
+        lr.long_list[atomicAdd(&lr.counters[1], 1u)] = (int32_t)row;
+      else
+        lr.mid_list[atomicAdd(&lr.counters[0], 1u)] = (int32_t)row;
     }
     end = beg;
     row_ok = false;
@@ -394,7 +393,7 @@ spmm_long_rows_kernel(int64_t k, float alpha, const float* __restrict__ vals, co
   constexpr int CW = 128 * KV;   // columns per pass
   __shared__ __align__(16) float red[LR_WARPS][CW];
   __shared__ uint32_t ticket_s;
-  const uint32_t n_mid = lr.counters[0], n_long = min(lr.counters[1], (uint32_t)kLongCap);
+  const uint32_t n_mid = lr.counters[0], n_long = lr.counters[1];
   if (n_mid == 0 && n_long == 0) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t base = offs[0];
@@ -647,7 +646,7 @@ int spmm_vec_launch(bof_ctx* ctx, cudaStream_t s, int64_t m, int64_t k, float al
   constexpr int ROWS_PER_BLOCK = 8 * (32 / L);
   dim3 grid((unsigned)ceil_div<int64_t>(m, ROWS_PER_BLOCK),
             (unsigned)ceil_div<int64_t>(k, 4 * L * KV));
-  // state of the deferred-row path: [counters 256 B | long_list | partials G x 512 floats | mid_list m entries]
+  // state of the deferred-row path: [counters 256 B | long_list m_cap | partials G x 512 floats | mid_list m_cap]
   static const bool defer = getenv("BOF_SPMM_NO_SPLIT") == nullptr;
   LongRows lr{nullptr, nullptr, nullptr};
   float* partial_ws = nullptr;
@@ -665,7 +664,7 @@ int spmm_vec_launch(bof_ctx* ctx, cudaStream_t s, int64_t m, int64_t k, float al
       lgrid = ctx->num_sms * std::min(per_sm, 2);   // co-resident by construction: the grid barrier relies on it
       size_t m_cap = 1024;
       while ((int64_t)m_cap < m) m_cap <<= 1;       // power-of-two sizing: a streamed pipeline regrows the slot rarely
-      const size_t bytes = 256 + (size_t)kLongCap * 4 + (size_t)lgrid * 512 * 4 + m_cap * 4;
+      const size_t bytes = 256 + m_cap * 4 + (size_t)lgrid * 512 * 4 + m_cap * 4;
       void* p = nullptr;
       const size_t had = ctx->slot_bytes[kSlotSpmmLong];
       { const int rc_slot = slot_reserve(ctx, kSlotSpmmLong, bytes, &p); if (rc_slot != BOF_OK) return rc_slot; }
@@ -674,8 +673,8 @@ int spmm_vec_launch(bof_ctx* ctx, cudaStream_t s, int64_t m, int64_t k, float al
       uint8_t* b8 = static_cast<uint8_t*>(p);
       lr.counters = reinterpret_cast<uint32_t*>(b8);
       lr.long_list = reinterpret_cast<int32_t*>(b8 + 256);
-      partial_ws = reinterpret_cast<float*>(b8 + 256 + (size_t)kLongCap * 4);
-      lr.mid_list = reinterpret_cast<int32_t*>(b8 + 256 + (size_t)kLongCap * 4 + (size_t)lgrid * 512 * 4);
+      partial_ws = reinterpret_cast<float*>(b8 + 256 + m_cap * 4);
+      lr.mid_list = reinterpret_cast<int32_t*>(b8 + 256 + m_cap * 4 + (size_t)lgrid * 512 * 4);
     } else {
       cudaGetLastError();
     }
