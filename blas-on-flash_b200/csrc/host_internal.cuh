@@ -95,7 +95,4 @@ int comm_push(bof_ctx* ctx, size_t offset, size_t count, int item, cudaEvent_t r
 int comm_wait_item(bof_ctx* ctx, cudaStream_t s, int item);
 void comm_sync_pushes(bof_ctx* ctx);
 
-// ---- sparse_host.cu ----
-std::vector<int64_t> partition_rows(const int64_t* ia, int64_t m, int64_t max_nnz);
-
 }  // namespace bof

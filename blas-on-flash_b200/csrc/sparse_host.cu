@@ -3,11 +3,31 @@
 // src/blas/csrcsc.cpp, include/tasks/{csrmm,csrgemv,csrcsc}_task.h.
 #include "host_internal.cuh"
 
+#include <memory>
+
 namespace bof {
+
+constexpr cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
+
+// Event ids of the sparse host calls: + g per block generation, + gp per B panel, + q per piece of an exchanged B.
+// No two of these calls run at once, so bof_csr_mm and csrcsc reuse the numbers of the streamed csrmm.
+constexpr int kBPieces = 4;  // pieces of a rank's own rows of an exchanged B
+enum SparseEvent : int {
+  EV_B = 0,                              // dense operand uploaded (B of csrmm, x of csrgemv)
+  EV_A = 1,                              // csrmm('T'): A uploaded for the device transpose
+  EV_C0 = 2,                             // csrmm('T'): old C uploaded
+  EV_UP = 4, EV_DONE = 6, EV_DOWN = 8,   // inputs of a block uploaded; its C rows computed; its C rows downloaded
+  EV_PIECE = 100,                        // collective csrmm: own piece q of B uploaded
+  EV_PAN = 0, EV_PAN_FREE = 2,           // bof_csr_mm: B panel uploaded; B panel consumed
+  EV_CSC_A = 0, EV_CSC_T = 1,            // csrcsc: A uploaded; A^T built and widened
+};
+static_assert(EV_B < EV_A && EV_A < EV_C0 && EV_C0 < EV_UP && EV_UP + 2 <= EV_DONE && EV_DONE + 2 <= EV_DOWN &&
+              EV_DOWN + 2 <= EV_PIECE, "csrmm / csrgemv: event ranges overlap");
+static_assert(EV_PAN + 2 <= EV_PAN_FREE && EV_PAN_FREE + 2 <= EV_UP, "bof_csr_mm: event ranges overlap");
 
 // Row-block partition by nnz budget (the idea of get_next_blk_size, include/blas_utils.h:72-82):
 // blocks[i] .. blocks[i+1] are the rows of block i.
-std::vector<int64_t> partition_rows(const int64_t* ia, int64_t m, int64_t max_nnz) {
+static std::vector<int64_t> partition_rows(const int64_t* ia, int64_t m, int64_t max_nnz) {
   std::vector<int64_t> cuts{0};
   int64_t r = 0;
   while (r < m) {
@@ -20,6 +40,246 @@ std::vector<int64_t> partition_rows(const int64_t* ia, int64_t m, int64_t max_nn
   return cuts;
 }
 
+// A CSR matrix on the device with int32 column indices.
+struct DevCsr { const int64_t* offs; const int32_t* idx; const float* vals; };
+
+// The row blocks in which csrmm('N') and csrgemv stream A: block i is rows [cuts[i], cuts[i + 1]) and lands in
+// generation i & 1 of the device buffers, which are sized for the largest block.
+struct RowBlocks {
+  std::vector<int64_t> cuts;
+  int64_t max_rows = 1, max_nnz = 1;
+  int64_t* offs[2]; int64_t* idx64[2]; int32_t* idx32[2]; float* vals[2];
+  int count() const { return (int)cuts.size() - 1; }
+};
+
+static int plan_row_blocks(bof_ctx* ctx, const int64_t* ia, int64_t m, RowBlocks* rb) {
+  const int64_t nnz = ia[m] - ia[0];
+  int64_t budget = (int64_t)ctx->cfg.csrmm_max_nnz;
+  budget = std::min(budget, std::max<int64_t>(nnz / 8, 1 << 20));  // >= 8 blocks when the matrix is big enough
+  rb->cuts = partition_rows(ia, m, budget);
+  for (int i = 0; i < rb->count(); ++i) {
+    rb->max_rows = std::max(rb->max_rows, rb->cuts[i + 1] - rb->cuts[i]);
+    rb->max_nnz = std::max(rb->max_nnz, ia[rb->cuts[i + 1]] - ia[rb->cuts[i]]);
+  }
+  for (int g = 0; g < 2; ++g) {
+    BOF_TRY(slot_reserve(ctx, S_OFFS + g, (size_t)rb->max_rows + 1, &rb->offs[g]));
+    BOF_TRY(slot_reserve(ctx, S_IDX64 + g, (size_t)rb->max_nnz, &rb->idx64[g]));
+    BOF_TRY(slot_reserve(ctx, S_IDX32 + g, (size_t)rb->max_nnz, &rb->idx32[g]));
+    BOF_TRY(slot_reserve(ctx, S_VALS + g, (size_t)rb->max_nnz, &rb->vals[g]));
+  }
+  return BOF_OK;
+}
+
+// Block i of A into its generation on the h2d stream; the caller narrows its indices once they have landed.
+static int upload_a_block(bof_ctx* ctx, const RowBlocks& rb, int i, const float* a, const int64_t* ia, const int64_t* ja) {
+  const int g = i & 1;
+  const int64_t r0 = rb.cuts[i], r1 = rb.cuts[i + 1], z0 = ia[r0] - ia[0], bnnz = ia[r1] - ia[r0];
+  BOF_TRY(copy1d(ctx, rb.offs[g], ia + r0, (size_t)(r1 - r0 + 1) * 8, H2D, ctx->h2d));
+  BOF_TRY(copy1d(ctx, rb.idx64[g], ja + z0, (size_t)bnnz * 8, H2D, ctx->h2d));
+  return copy1d(ctx, rb.vals[g], a + z0, (size_t)bnnz * 4, H2D, ctx->h2d);
+}
+
+// A^T of the device CSR A [m x n] into (offs_t, idx_t, vals_t) on the compute stream, with its workspace in S_WS.
+static int transpose_csr(bof_ctx* ctx, int64_t m, int64_t n, int64_t nnz, const int64_t* offs, const int32_t* idx,
+                         const float* vals, int64_t* offs_t, int32_t* idx_t, float* vals_t) {
+  void* ws;
+  const size_t wsb = csr2csc_workspace_bytes(m, n, nnz);
+  BOF_TRY(slot_reserve(ctx, S_WS, wsb, &ws));
+  return launch_csr2csc(ctx, ctx->compute, m, n, nnz, offs, idx, vals, offs_t, idx_t, vals_t, ws, wsb);
+}
+
+// A^T (K6) of the host CSR A [m x n] in S_OUT0..2: A is uploaded whole (event ev_up), narrowed and transposed on the
+// compute stream.  Its int64 indices are staged in S_IDX64, which is free again once the transpose has run.
+static int upload_transposed(bof_ctx* ctx, int64_t m, int64_t n, int64_t nnz, const float* a, const int64_t* ia,
+                             const int64_t* ja, int ev_up, DevCsr* at) {
+  const size_t z = (size_t)std::max<int64_t>(nnz, 1);
+  int64_t *offs_d, *offs_t, *idx64;
+  int32_t *idx32, *idx_t;
+  float *vals_d, *vals_t;
+  BOF_TRY(slot_reserve(ctx, S_OFFS, (size_t)m + 1, &offs_d));
+  BOF_TRY(slot_reserve(ctx, S_IDX64, z, &idx64));
+  BOF_TRY(slot_reserve(ctx, S_IDX32, z, &idx32));
+  BOF_TRY(slot_reserve(ctx, S_VALS, z, &vals_d));
+  BOF_TRY(slot_reserve(ctx, S_OUT0, (size_t)n + 1, &offs_t));
+  BOF_TRY(slot_reserve(ctx, S_OUT1, z, &idx_t));
+  BOF_TRY(slot_reserve(ctx, S_OUT2, z, &vals_t));
+  BOF_TRY(copy1d(ctx, offs_d, ia, (size_t)(m + 1) * 8, H2D, ctx->h2d));
+  BOF_TRY(copy1d(ctx, idx64, ja, (size_t)nnz * 8, H2D, ctx->h2d));
+  BOF_TRY(copy1d(ctx, vals_d, a, (size_t)nnz * 4, H2D, ctx->h2d));
+  BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, ev_up), ctx->h2d));
+  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, ev_up), 0));
+  BOF_TRY(launch_idx_narrow(ctx, ctx->compute, idx64, idx32, nnz));
+  BOF_TRY(transpose_csr(ctx, m, n, nnz, offs_d, idx32, vals_d, offs_t, idx_t, vals_t));
+  *at = DevCsr{offs_t, idx_t, vals_t};
+  return BOF_OK;
+}
+
+// Host C of a csrmm: row-major with pitch ld, or column-major with pitch ld (its row count).  The block of rows
+// [r0, r0 + rows) x columns [j0, j0 + w) lies on the device tight: [rows x w], or [w x rows] for a column-major C.
+struct HostC { float* c; int64_t ld; bool colmaj; };
+
+static int upload_c_block(bof_ctx* ctx, const HostC& hc, int64_t r0, int64_t rows, int64_t j0, int64_t w, float* blk) {
+  if (hc.colmaj)
+    return copy2d(ctx, blk, (size_t)rows * 4, hc.c + j0 * hc.ld + r0, (size_t)hc.ld * 4, (size_t)rows * 4, (size_t)w, H2D, ctx->h2d);
+  return copy2d(ctx, blk, (size_t)w * 4, hc.c + r0 * hc.ld + j0, (size_t)hc.ld * 4, (size_t)w * 4, (size_t)rows, H2D, ctx->h2d);
+}
+
+// The same block from the device to the host C, on the d2h stream (see d2h_transfer for the events and the ticket).
+static int download_c_block(bof_ctx* ctx, const HostC& hc, int64_t r0, int64_t rows, int64_t j0, int64_t w,
+                            const float* blk, cudaEvent_t wait_ev, cudaEvent_t record_ev, uint64_t* ticket) {
+  if (hc.colmaj)
+    return d2h_transfer(ctx, hc.c + j0 * hc.ld + r0, (size_t)hc.ld * 4, blk, (size_t)rows * 4, (size_t)rows * 4, (size_t)w,
+                        ctx->d2h, wait_ev, record_ev, ticket);
+  return d2h_transfer(ctx, hc.c + r0 * hc.ld + j0, (size_t)hc.ld * 4, blk, (size_t)w * 4, (size_t)w * 4, (size_t)rows,
+                      ctx->d2h, wait_ev, record_ev, ticket);
+}
+
+// C block [rows x w] = alpha A_blk B + beta C block on the compute stream, B [b_rows x w] row-major.  A column-major
+// C (cblk_t != nullptr) is computed into cblk and transposed into cblk_t [w x rows], which holds the old C block.
+static int spmm_c_block(bof_ctx* ctx, int64_t rows, int64_t w, float alpha, const DevCsr& a, const float* B,
+                        int64_t b_rows, float beta, float* cblk, float* cblk_t) {
+  if (cblk_t == nullptr)
+    return launch_spmm_rm(ctx, ctx->compute, rows, w, alpha, a.vals, a.idx, a.offs, B, w, beta, cblk, w, b_rows);
+  BOF_TRY(launch_spmm_rm(ctx, ctx->compute, rows, w, 1.f, a.vals, a.idx, a.offs, B, w, 0.f, cblk, w, b_rows));
+  return launch_transpose_axpby(ctx, ctx->compute, rows, w, alpha, cblk, w, beta, cblk_t, rows);
+}
+
+// bof_dist_csrmm: B [in_rows x k] is replicated over the ranks.  Every rank uploads rows [r0, r1) of it (1/world of
+// the PCIe traffic) in a few pieces and pushes each piece into every peer's exchange buffer Bd with copy-engine peer
+// copies over NVLink as soon as it has landed; meanwhile this rank's first A blocks upload behind the slice.  The
+// SpMM gathers arbitrary rows of B, so the compute stream waits for every piece of every rank.
+static int exchange_dense(bof_ctx* ctx, const float* b, int64_t in_rows, int64_t k, float* Bd) {
+  const int world = comm_world(ctx), rank = comm_rank(ctx);
+  auto piece = [&](int r, int q, int64_t* p0, int64_t* p1) {   // rows [p0, p1) of B: piece q of rank r's shard
+    const int64_t base = in_rows / world, rem = in_rows % world;
+    const int64_t r0 = r * base + std::min<int64_t>(r, rem), r1 = r0 + base + (r < rem ? 1 : 0);
+    const int64_t per = ceil_div<int64_t>(r1 - r0, kBPieces);
+    *p0 = std::min(r1, r0 + q * per);
+    *p1 = std::min(r1, *p0 + per);
+  };
+  for (int q = 0; q < kBPieces; ++q) {
+    int64_t p0, p1;
+    piece(rank, q, &p0, &p1);
+    if (p1 <= p0) continue;
+    BOF_TRY(copy1d(ctx, Bd + p0 * k, b + p0 * k, (size_t)(p1 - p0) * k * 4, H2D, ctx->h2d));
+    cudaEvent_t ev_own = get_event(ctx, EV_PIECE + q);
+    BOF_CUDA(ctx, cudaEventRecord(ev_own, ctx->h2d));
+    BOF_TRY(comm_push(ctx, (size_t)(p0 * k), (size_t)(p1 - p0) * k, rank * kBPieces + q, ev_own));
+    if (q == kBPieces - 1) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_own, 0));
+  }
+  trace_mark(ctx, ctx->h2d, "h2d: own slice of the dense operand landed", rank);
+  for (int src = 0; src < world; ++src) {
+    if (src == rank) continue;
+    for (int q = 0; q < kBPieces; ++q) {
+      int64_t p0, p1;
+      piece(src, q, &p0, &p1);
+      if (p1 > p0) BOF_TRY(comm_wait_item(ctx, ctx->compute, src * kBPieces + q));
+    }
+  }
+  trace_mark(ctx, ctx->compute, "compute: dense operand complete on this rank", 0);
+  return BOF_OK;
+}
+
+// csrmm's B [in_rows x k] row-major on the device for the compute stream: b_dev as it is, exchanged by a collective
+// call, or uploaded from a host B, column-major or row-major with pitch ldb.
+static int upload_dense(bof_ctx* ctx, const float* b, const float* b_dev, bool collective, bool colmaj, int64_t in_rows,
+                        int64_t k, int64_t ldb, float** Bd) {
+  if (b_dev != nullptr) {
+    *Bd = const_cast<float*>(b_dev);  // already in HBM (e.g. all-gathered over NVLink); read-only here
+    return BOF_OK;
+  }
+  if (collective) {
+    BOF_TRY(comm_exchange_begin(ctx, (size_t)in_rows * k * sizeof(float), Bd));   // the buffer the peers push into
+    return exchange_dense(ctx, b, in_rows, k, *Bd);
+  }
+  BOF_TRY(slot_reserve(ctx, S_DENSE, (size_t)in_rows * k, Bd));
+  float* Braw = nullptr;
+  if (colmaj) {
+    BOF_TRY(slot_reserve(ctx, S_DENSE_T, (size_t)in_rows * k, &Braw));
+    BOF_TRY(copy1d(ctx, Braw, b, (size_t)in_rows * k * 4, H2D, ctx->h2d));
+  } else {
+    BOF_TRY(copy2d(ctx, *Bd, (size_t)k * 4, b, (size_t)ldb * 4, (size_t)k * 4, (size_t)in_rows, H2D, ctx->h2d));
+  }
+  BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_B), ctx->h2d));
+  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_B), 0));
+  if (colmaj) BOF_TRY(launch_transpose(ctx, ctx->compute, k, in_rows, Braw, in_rows, *Bd, k));
+  return BOF_OK;
+}
+
+// csrmm('T'): A^T in CSR on the device, then the no-transpose kernel on its n rows into the whole C [n x k] on the
+// device (beta needs the old C).
+static int csrmm_transposed(bof_ctx* ctx, int64_t m, int64_t n, int64_t k, float alpha, float beta, const float* a,
+                            const int64_t* ia, const int64_t* ja, const float* Bd, float* c, bool colmaj) {
+  const int64_t nnz = ia[m] - ia[0];
+  BOF_REQUIRE(ctx, nnz < (1ll << 31), "csrmm('T'): nnz must be below 2^31");
+  DevCsr at;
+  BOF_TRY(upload_transposed(ctx, m, n, nnz, a, ia, ja, EV_A, &at));
+  float *Cd, *Ccm = nullptr;
+  BOF_TRY(slot_reserve(ctx, S_CBLK, (size_t)n * k, &Cd));
+  if (colmaj) BOF_TRY(slot_reserve(ctx, S_CBLK_T, (size_t)n * k, &Ccm));
+  float* Cio = colmaj ? Ccm : Cd;  // what is copied from/to the host
+  if (beta != 0.f) {
+    BOF_TRY(copy1d(ctx, Cio, c, (size_t)n * k * 4, H2D, ctx->h2d));
+    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_C0), ctx->h2d));
+    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_C0), 0));
+  }
+  BOF_TRY(spmm_c_block(ctx, n, k, alpha, at, Bd, m, beta, Cd, Ccm));
+  BOF_TRY(copy1d(ctx, c, Cio, (size_t)n * k * 4, D2H, ctx->compute));
+  return sync_all(ctx);
+}
+
+// csrmm('N'): A streams in row blocks, C block by block.  Software-pipelined issue order: block i+1 is uploaded and
+// launched before block i is downloaded, so a (host-blocking) staged download of block i overlaps the kernel of
+// block i+1 and the copy engines never wait on the host.
+static int csrmm_streamed(bof_ctx* ctx, int64_t m, int64_t n, int64_t k, float alpha, float beta, const float* a,
+                          const int64_t* ia, const int64_t* ja, const float* Bd, const HostC& hc) {
+  RowBlocks rb;
+  BOF_TRY(plan_row_blocks(ctx, ia, m, &rb));
+  float* cblk[2]; float* cblk_t[2] = {nullptr, nullptr};
+  for (int g = 0; g < 2; ++g) {
+    BOF_TRY(slot_reserve(ctx, S_CBLK + g, (size_t)rb.max_rows * k, &cblk[g]));
+    if (hc.colmaj) BOF_TRY(slot_reserve(ctx, S_CBLK_T + g, (size_t)rb.max_rows * k, &cblk_t[g]));
+  }
+  bool used[2] = {false, false};
+  uint64_t down_ticket[2] = {0, 0};  // pageable C: the drainer enqueues the download and records ev_down
+  auto stage_block = [&](int i) -> int {
+    const int g = i & 1;
+    const int64_t r0 = rb.cuts[i], r1 = rb.cuts[i + 1], rows = r1 - r0;
+    cudaEvent_t ev_up = get_event(ctx, EV_UP + g), ev_done = get_event(ctx, EV_DONE + g), ev_down = get_event(ctx, EV_DOWN + g);
+    if (used[g]) {
+      d2h_fence(ctx, down_ticket[g]);  // ev_down of block i-2 has been recorded (and ev_done may be re-recorded)
+      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_done, 0));   // inputs of block i-2 consumed
+      // Only an upload of old C rows (beta != 0) touches the C buffer from this stream; waiting for the download
+      // unconditionally idled the H2D engine ~9 ms every other block (BOF_TRACE timeline, cfg-3: 419 -> 37x ms).
+      if (beta != 0.f) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_down, 0));   // its C rows left the device
+    }
+    BOF_TRY(upload_a_block(ctx, rb, i, a, ia, ja));
+    if (beta != 0.f) BOF_TRY(upload_c_block(ctx, hc, r0, rows, 0, k, hc.colmaj ? cblk_t[g] : cblk[g]));
+    BOF_CUDA(ctx, cudaEventRecord(ev_up, ctx->h2d));
+    trace_mark(ctx, ctx->h2d, "h2d: A block landed", i);
+    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_up, 0));
+    if (used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_down, 0));
+    trace_mark(ctx, ctx->compute, "compute: block start", i);
+    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, rb.idx64[g], rb.idx32[g], ia[r1] - ia[r0]));
+    BOF_TRY(spmm_c_block(ctx, rows, k, alpha, DevCsr{rb.offs[g], rb.idx32[g], rb.vals[g]}, Bd, n, beta, cblk[g], cblk_t[g]));
+    BOF_CUDA(ctx, cudaEventRecord(ev_done, ctx->compute));
+    trace_mark(ctx, ctx->compute, "compute: block end", i);
+    used[g] = true;
+    return BOF_OK;
+  };
+  const int nblk = rb.count();
+  if (nblk > 0) BOF_TRY(stage_block(0));
+  for (int i = 0; i < nblk; ++i) {
+    if (i + 1 < nblk) BOF_TRY(stage_block(i + 1));
+    const int g = i & 1;
+    BOF_TRY(download_c_block(ctx, hc, rb.cuts[i], rb.cuts[i + 1] - rb.cuts[i], 0, k, hc.colmaj ? cblk_t[g] : cblk[g],
+                             get_event(ctx, EV_DONE + g), get_event(ctx, EV_DOWN + g), &down_ticket[g]));
+    trace_mark(ctx, ctx->d2h, "d2h: C block downloaded", i);
+  }
+  BOF_TRY(sync_all(ctx));
+  trace_dump(ctx, "bof_host_csrmm");
+  return BOF_OK;
+}
 
 }  // namespace bof
 
@@ -46,222 +306,18 @@ static int host_csrmm_impl(bof_ctx* ctx, char trans_a, int64_t m, int64_t n, int
   const int64_t out_rows = trans_a == 'N' ? m : n;   // rows of C
   const int64_t in_rows = trans_a == 'N' ? n : m;    // rows of B
   // a collective call (bof_dist_csrmm) exchanges the dense operand on every rank, also on one that owns no rows of C
-  const bool dist_mode = dist_b && comm_world(ctx) > 1;
-  if (k == 0 || (out_rows == 0 && !dist_mode)) { stats_end(ctx); return call_guard.done(); }
+  const bool collective = dist_b && comm_world(ctx) > 1;
+  if (k == 0 || (out_rows == 0 && !collective)) { stats_end(ctx); return call_guard.done(); }
   const bool colmaj = ord_b == 'C';
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
-
-  // resident dense operand, always row-major [in_rows x k] on the device
   float* Bd = nullptr;
-  if (b_dev != nullptr) {
-    Bd = const_cast<float*>(b_dev);  // already in HBM (e.g. all-gathered over NVLink); read-only here
-  } else if (dist_mode) {
-    BOF_TRY(comm_exchange_begin(ctx, (size_t)in_rows * k * sizeof(float), &Bd));   // the buffer the peers push into
-  } else {
-    BOF_TRY(slot_reserve(ctx, S_DENSE, (size_t)in_rows * k, &Bd));
-  }
-  const int world = dist_b ? comm_world(ctx) : 1, rank = comm_rank(ctx);
-  if (b_dev != nullptr) {
-    // nothing to upload
-  } else if (dist_mode) {
-    // bof_dist_csrmm: B is replicated over the ranks.  Every rank uploads rows [r0, r1) of it (1/world of the PCIe
-    // traffic) in a few pieces and pushes each piece into every peer's exchange buffer with copy-engine peer copies
-    // over NVLink as soon as it has landed; meanwhile this rank's first A blocks upload behind the slice.  The SpMM
-    // gathers arbitrary rows of B, so the compute stream waits for every piece of every rank.
-    constexpr int kPieces = 4;
-    auto shard = [&](int r, int64_t* r0, int64_t* r1) {
-      const int64_t base = in_rows / world, rem = in_rows % world;
-      *r0 = r * base + std::min<int64_t>(r, rem);
-      *r1 = *r0 + base + (r < rem ? 1 : 0);
-    };
-    auto piece = [&](int r, int q, int64_t* p0, int64_t* p1) {
-      int64_t r0, r1;
-      shard(r, &r0, &r1);
-      const int64_t per = ceil_div<int64_t>(r1 - r0, kPieces);
-      *p0 = std::min(r1, r0 + q * per);
-      *p1 = std::min(r1, *p0 + per);
-    };
-    for (int q = 0; q < kPieces; ++q) {
-      int64_t p0, p1;
-      piece(rank, q, &p0, &p1);
-      if (p1 <= p0) continue;
-      BOF_TRY(copy1d(ctx, Bd + p0 * k, b + p0 * k, (size_t)(p1 - p0) * k * 4, H2D, ctx->h2d));
-      cudaEvent_t ev_own = get_event(ctx, 100 + q);
-      BOF_CUDA(ctx, cudaEventRecord(ev_own, ctx->h2d));
-      BOF_TRY(comm_push(ctx, (size_t)(p0 * k), (size_t)(p1 - p0) * k, rank * kPieces + q, ev_own));
-      if (q == kPieces - 1) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_own, 0));
-    }
-    trace_mark(ctx, ctx->h2d, "h2d: own slice of the dense operand landed", rank);
-    for (int src = 0; src < world; ++src) {
-      if (src == rank) continue;
-      for (int q = 0; q < kPieces; ++q) {
-        int64_t p0, p1;
-        piece(src, q, &p0, &p1);
-        if (p1 > p0) BOF_TRY(comm_wait_item(ctx, ctx->compute, src * kPieces + q));
-      }
-    }
-    trace_mark(ctx, ctx->compute, "compute: dense operand complete on this rank", 0);
-  } else if (colmaj) {
-    float* Braw = nullptr;
-    BOF_TRY(slot_reserve(ctx, S_DENSE_T, (size_t)in_rows * k, &Braw));
-    BOF_TRY(copy1d(ctx, Braw, b, (size_t)in_rows * k * 4, H2D, ctx->h2d));
-    cudaEvent_t evB = get_event(ctx, 0);
-    BOF_CUDA(ctx, cudaEventRecord(evB, ctx->h2d));
-    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, evB, 0));
-    BOF_TRY(launch_transpose(ctx, ctx->compute, k, in_rows, Braw, in_rows, Bd, k));
-  } else {
-    BOF_TRY(copy2d(ctx, Bd, (size_t)k * 4, b, (size_t)ldk * 4, (size_t)k * 4, (size_t)in_rows, H2D, ctx->h2d));
-    cudaEvent_t evB = get_event(ctx, 0);
-    BOF_CUDA(ctx, cudaEventRecord(evB, ctx->h2d));
-    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, evB, 0));
-  }
-
+  BOF_TRY(upload_dense(ctx, b, b_dev, collective, colmaj, in_rows, k, ldk, &Bd));
   if (out_rows == 0) {   // collective call, empty shard: my slice has been pushed and the peers' slices have arrived
     BOF_TRY(sync_all(ctx));
-    stats_end(ctx);
-    return call_guard.done();
+  } else {
+    trace_mark(ctx, ctx->h2d, "h2d: dense operand landed", 0);
+    if (trans_a == 'T') BOF_TRY(csrmm_transposed(ctx, m, n, k, alpha, beta, a, ia, ja, Bd, c, colmaj));
+    else BOF_TRY(csrmm_streamed(ctx, m, n, k, alpha, beta, a, ia, ja, Bd, HostC{c, colmaj ? m : ldk, colmaj}));
   }
-  trace_mark(ctx, ctx->h2d, "h2d: dense operand landed", 0);
-  const int64_t* offs_host = ia;
-  const int64_t nnz = ia[m] - ia[0];
-  std::vector<int64_t> tr_offs_host;  // only for 'T'
-  const int32_t* idx_dev_all = nullptr;  // 'T': transposed matrix resident on the device
-  const float* vals_dev_all = nullptr;
-  const int64_t* offs_dev_all = nullptr;
-
-  if (trans_a == 'T') {
-    // A^T in CSR on the device (K6), then the no-transpose kernel on n rows.
-    BOF_REQUIRE(ctx, nnz < (1ll << 31), "csrmm('T'): nnz must be below 2^31");
-    int64_t *offs_d, *offs_t, *idx64;
-    int32_t *idx32, *idx_t;
-    float *vals_d, *vals_t;
-    void* ws;
-    const size_t wsb = csr2csc_workspace_bytes(m, n, nnz);
-    BOF_TRY(slot_reserve(ctx, S_OFFS, (size_t)m + 1, &offs_d));
-    BOF_TRY(slot_reserve(ctx, S_IDX64, (size_t)std::max<int64_t>(nnz, 1), &idx64));
-    BOF_TRY(slot_reserve(ctx, S_IDX32, (size_t)std::max<int64_t>(nnz, 1), &idx32));
-    BOF_TRY(slot_reserve(ctx, S_VALS, (size_t)std::max<int64_t>(nnz, 1), &vals_d));
-    BOF_TRY(slot_reserve(ctx, S_OUT0, (size_t)n + 1, &offs_t));
-    BOF_TRY(slot_reserve(ctx, S_OUT1, (size_t)std::max<int64_t>(nnz, 1), &idx_t));
-    BOF_TRY(slot_reserve(ctx, S_OUT2, (size_t)std::max<int64_t>(nnz, 1), &vals_t));
-    BOF_TRY(slot_reserve(ctx, S_WS, wsb, &ws));
-    BOF_TRY(copy1d(ctx, offs_d, ia, (size_t)(m + 1) * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, idx64, ja, (size_t)nnz * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, vals_d, a, (size_t)nnz * 4, H2D, ctx->h2d));
-    cudaEvent_t ev = get_event(ctx, 1);
-    BOF_CUDA(ctx, cudaEventRecord(ev, ctx->h2d));
-    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev, 0));
-    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, idx64, idx32, nnz));
-    BOF_TRY(launch_csr2csc(ctx, ctx->compute, m, n, nnz, offs_d, idx32, vals_d, offs_t, idx_t, vals_t, ws, wsb));
-    offs_dev_all = offs_t;
-    idx_dev_all = idx_t;
-    vals_dev_all = vals_t;
-  }
-
-  if (trans_a == 'T') {
-    // whole C on the device (n x k); beta needs the old C
-    float* Cd = nullptr;
-    BOF_TRY(slot_reserve(ctx, S_CBLK, (size_t)out_rows * k, &Cd));
-    float* Cio = Cd;  // what is copied from/to the host
-    float* Ccm = nullptr;
-    if (colmaj) { BOF_TRY(slot_reserve(ctx, S_CBLK_T, (size_t)out_rows * k, &Ccm)); Cio = Ccm; }
-    if (beta != 0.f) {
-      BOF_TRY(copy1d(ctx, Cio, c, (size_t)out_rows * k * 4, H2D, ctx->h2d));
-      cudaEvent_t ev = get_event(ctx, 2);
-      BOF_CUDA(ctx, cudaEventRecord(ev, ctx->h2d));
-      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev, 0));
-    }
-    if (colmaj) {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, out_rows, k, 1.f, vals_dev_all, idx_dev_all, offs_dev_all, Bd, k, 0.f, Cd, k, in_rows));
-      BOF_TRY(launch_transpose_axpby(ctx, ctx->compute, out_rows, k, alpha, Cd, k, beta, Ccm, out_rows));
-    } else {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, out_rows, k, alpha, vals_dev_all, idx_dev_all, offs_dev_all, Bd, k, beta, Cd, k, in_rows));
-    }
-    BOF_TRY(copy1d(ctx, c, Cio, (size_t)out_rows * k * 4, D2H, ctx->compute));
-    BOF_TRY(sync_all(ctx));
-    stats_end(ctx);
-    return call_guard.done();
-  }
-
-  // ---- 'N': streamed row blocks ----
-  int64_t budget = (int64_t)ctx->cfg.csrmm_max_nnz;
-  budget = std::min(budget, std::max<int64_t>(nnz / 8, 1 << 20));  // >= 8 blocks when the matrix is big enough
-  const std::vector<int64_t> cuts = partition_rows(offs_host, m, budget);
-  const int nblk = (int)cuts.size() - 1;
-  int64_t max_rows = 1, max_nnz = 1;
-  for (int i = 0; i < nblk; ++i) {
-    max_rows = std::max(max_rows, cuts[i + 1] - cuts[i]);
-    max_nnz = std::max(max_nnz, offs_host[cuts[i + 1]] - offs_host[cuts[i]]);
-  }
-  int64_t* offs_d[2]; int64_t* idx64_d[2]; int32_t* idx32_d[2]; float* vals_d[2]; float* cblk[2]; float* cblk_t[2] = {nullptr, nullptr};
-  for (int g = 0; g < 2; ++g) {
-    BOF_TRY(slot_reserve(ctx, S_OFFS + g, (size_t)max_rows + 1, &offs_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_IDX64 + g, (size_t)max_nnz, &idx64_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_IDX32 + g, (size_t)max_nnz, &idx32_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_VALS + g, (size_t)max_nnz, &vals_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_CBLK + g, (size_t)max_rows * k, &cblk[g]));
-    if (colmaj) BOF_TRY(slot_reserve(ctx, S_CBLK_T + g, (size_t)max_rows * k, &cblk_t[g]));
-  }
-  // events: 4+g uploaded, 6+g computed, 8+g downloaded.  Software-pipelined issue order: block i+1 is
-  // uploaded and launched before block i is downloaded, so a (host-blocking) staged download of
-  // block i overlaps the kernel of block i+1 and the copy engines never wait on the host.
-  bool used[2] = {false, false};
-  uint64_t down_ticket[2] = {0, 0};  // pageable C: the drainer enqueues the download and records ev_down
-  auto stage_block = [&](int i) -> int {
-    const int g = i & 1;
-    const int64_t r0 = cuts[i], r1 = cuts[i + 1], rows = r1 - r0;
-    const int64_t z0 = offs_host[r0] - offs_host[0], z1 = offs_host[r1] - offs_host[0], bnnz = z1 - z0;
-    cudaEvent_t ev_up = get_event(ctx, 4 + g), ev_done = get_event(ctx, 6 + g), ev_down = get_event(ctx, 8 + g);
-    if (used[g]) {
-      d2h_fence(ctx, down_ticket[g]);  // ev_down of block i-2 has been recorded (and ev_done may be re-recorded)
-      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_done, 0));   // inputs of block i-2 consumed
-      // Only an upload of old C rows (beta != 0) touches the C buffer from this stream; waiting for the download
-      // unconditionally idled the H2D engine ~9 ms every other block (BOF_TRACE timeline, cfg-3: 419 -> 37x ms).
-      if (beta != 0.f) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_down, 0));   // its C rows left the device
-    }
-    BOF_TRY(copy1d(ctx, offs_d[g], offs_host + r0, (size_t)(rows + 1) * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, idx64_d[g], ja + z0, (size_t)bnnz * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, vals_d[g], a + z0, (size_t)bnnz * 4, H2D, ctx->h2d));
-    float* c_io = colmaj ? cblk_t[g] : cblk[g];
-    if (beta != 0.f) {
-      if (colmaj) BOF_TRY(copy2d(ctx, c_io, (size_t)rows * 4, c + r0, (size_t)m * 4, (size_t)rows * 4, (size_t)k, H2D, ctx->h2d));
-      else BOF_TRY(copy2d(ctx, c_io, (size_t)k * 4, c + r0 * ldk, (size_t)ldk * 4, (size_t)k * 4, (size_t)rows, H2D, ctx->h2d));
-    }
-    BOF_CUDA(ctx, cudaEventRecord(ev_up, ctx->h2d));
-    trace_mark(ctx, ctx->h2d, "h2d: A block landed", i);
-    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_up, 0));
-    if (used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_down, 0));
-    trace_mark(ctx, ctx->compute, "compute: block start", i);
-    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, idx64_d[g], idx32_d[g], bnnz));
-    if (colmaj) {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, rows, k, 1.f, vals_d[g], idx32_d[g], offs_d[g], Bd, k, 0.f, cblk[g], k, in_rows));
-      BOF_TRY(launch_transpose_axpby(ctx, ctx->compute, rows, k, alpha, cblk[g], k, beta, cblk_t[g], rows));
-    } else {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, rows, k, alpha, vals_d[g], idx32_d[g], offs_d[g], Bd, k, beta, cblk[g], k, in_rows));
-    }
-    BOF_CUDA(ctx, cudaEventRecord(ev_done, ctx->compute));
-    trace_mark(ctx, ctx->compute, "compute: block end", i);
-    used[g] = true;
-    return BOF_OK;
-  };
-  auto fetch_block = [&](int i) -> int {
-    const int g = i & 1;
-    const int64_t r0 = cuts[i], rows = cuts[i + 1] - r0;
-    float* c_io = colmaj ? cblk_t[g] : cblk[g];
-    cudaEvent_t ev_done = get_event(ctx, 6 + g), ev_down = get_event(ctx, 8 + g);
-    if (colmaj) BOF_TRY(d2h_transfer(ctx, c + r0, (size_t)m * 4, c_io, (size_t)rows * 4, (size_t)rows * 4, (size_t)k, ctx->d2h, ev_done, ev_down, &down_ticket[g]));
-    else if (ldk == k) BOF_TRY(d2h_transfer(ctx, c + r0 * k, (size_t)rows * k * 4, c_io, (size_t)rows * k * 4, (size_t)rows * k * 4, 1, ctx->d2h, ev_done, ev_down, &down_ticket[g]));
-    else BOF_TRY(d2h_transfer(ctx, c + r0 * ldk, (size_t)ldk * 4, c_io, (size_t)k * 4, (size_t)k * 4, (size_t)rows, ctx->d2h, ev_done, ev_down, &down_ticket[g]));
-    trace_mark(ctx, ctx->d2h, "d2h: C block downloaded", i);
-    return BOF_OK;
-  };
-  if (nblk > 0) BOF_TRY(stage_block(0));
-  for (int i = 0; i < nblk; ++i) {
-    if (i + 1 < nblk) BOF_TRY(stage_block(i + 1));
-    BOF_TRY(fetch_block(i));
-  }
-  BOF_TRY(sync_all(ctx));
-  trace_dump(ctx, "bof_host_csrmm");
   stats_end(ctx);
   return call_guard.done();
 }
@@ -326,7 +382,6 @@ int bof_host_csrgemv(bof_ctx* ctx, char trans_a, int64_t m, int64_t n, const flo
   BOF_CUDA(ctx, cudaSetDevice(ctx->device));
   stats_begin(ctx);
   CallGuard call_guard(ctx);
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
   const bool tr = trans_a == 'T';
   const int64_t xlen = tr ? m : n, ylen = tr ? n : m;
   if (ylen == 0) { stats_end(ctx); return call_guard.done(); }
@@ -334,49 +389,31 @@ int bof_host_csrgemv(bof_ctx* ctx, char trans_a, int64_t m, int64_t n, const flo
   BOF_TRY(slot_reserve(ctx, S_DENSE, (size_t)std::max<int64_t>(xlen, 1), &xd));
   BOF_TRY(slot_reserve(ctx, S_CBLK, (size_t)ylen, &yd));
   BOF_TRY(copy1d(ctx, xd, b, (size_t)xlen * 4, H2D, ctx->h2d));
-  cudaEvent_t evx = get_event(ctx, 0);
-  BOF_CUDA(ctx, cudaEventRecord(evx, ctx->h2d));
-  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, evx, 0));
+  BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_B), ctx->h2d));
+  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_B), 0));
   BOF_CUDA(ctx, cudaMemsetAsync(yd, 0, (size_t)ylen * 4, ctx->compute));
 
-  const int64_t nnz = ia[m] - ia[0];
-  int64_t budget = std::min<int64_t>((int64_t)ctx->cfg.csrmm_max_nnz, std::max<int64_t>(nnz / 8, 1 << 20));
-  const std::vector<int64_t> cuts = partition_rows(ia, m, budget);
-  const int nblk = (int)cuts.size() - 1;
-  int64_t max_rows = 1, max_nnz = 1;
-  for (int i = 0; i < nblk; ++i) {
-    max_rows = std::max(max_rows, cuts[i + 1] - cuts[i]);
-    max_nnz = std::max(max_nnz, ia[cuts[i + 1]] - ia[cuts[i]]);
-  }
-  int64_t* offs_d[2]; int64_t* idx64_d[2]; int32_t* idx32_d[2]; float* vals_d[2];
-  for (int g = 0; g < 2; ++g) {
-    BOF_TRY(slot_reserve(ctx, S_OFFS + g, (size_t)max_rows + 1, &offs_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_IDX64 + g, (size_t)max_nnz, &idx64_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_IDX32 + g, (size_t)max_nnz, &idx32_d[g]));
-    BOF_TRY(slot_reserve(ctx, S_VALS + g, (size_t)max_nnz, &vals_d[g]));
-  }
+  RowBlocks rb;
+  BOF_TRY(plan_row_blocks(ctx, ia, m, &rb));
   if (tr && ctx->cfg.spmv_t_atomic == 0) {   // workspace of the sorted A^T x path for the largest block, before the pipeline starts
     void* wsp = nullptr;
-    BOF_TRY(slot_reserve(ctx, kSlotSpmvT, spmv_t_workspace_bytes(n, max_nnz), &wsp));
+    BOF_TRY(slot_reserve(ctx, kSlotSpmvT, spmv_t_workspace_bytes(n, rb.max_nnz), &wsp));
   }
   bool used[2] = {false, false};
-  for (int i = 0; i < nblk; ++i) {
+  for (int i = 0; i < rb.count(); ++i) {
     const int g = i & 1;
-    const int64_t r0 = cuts[i], r1 = cuts[i + 1], rows = r1 - r0;
-    const int64_t z0 = ia[r0] - ia[0], bnnz = ia[r1] - ia[r0];
-    cudaEvent_t ev_up = get_event(ctx, 4 + g), ev_done = get_event(ctx, 6 + g);
+    const int64_t r0 = rb.cuts[i], r1 = rb.cuts[i + 1], rows = r1 - r0, bnnz = ia[r1] - ia[r0];
+    cudaEvent_t ev_up = get_event(ctx, EV_UP + g), ev_done = get_event(ctx, EV_DONE + g);
     if (used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_done, 0));
-    BOF_TRY(copy1d(ctx, offs_d[g], ia + r0, (size_t)(rows + 1) * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, idx64_d[g], ja + z0, (size_t)bnnz * 8, H2D, ctx->h2d));
-    BOF_TRY(copy1d(ctx, vals_d[g], a + z0, (size_t)bnnz * 4, H2D, ctx->h2d));
+    BOF_TRY(upload_a_block(ctx, rb, i, a, ia, ja));
     BOF_CUDA(ctx, cudaEventRecord(ev_up, ctx->h2d));
     BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_up, 0));
-    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, idx64_d[g], idx32_d[g], bnnz));
+    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, rb.idx64[g], rb.idx32[g], bnnz));
     if (!tr) {
-      BOF_TRY(launch_spmv(ctx, ctx->compute, 'N', rows, n, vals_d[g], idx32_d[g], offs_d[g], xd, yd + r0));
+      BOF_TRY(launch_spmv(ctx, ctx->compute, 'N', rows, n, rb.vals[g], rb.idx32[g], rb.offs[g], xd, yd + r0));
     } else {
       // y += A_blk^T x_blk : launch the accumulate kernel directly (y was zeroed once above)
-      BOF_TRY(launch_spmv(ctx, ctx->compute, 't', rows, n, vals_d[g], idx32_d[g], offs_d[g], xd + r0, yd, bnnz));
+      BOF_TRY(launch_spmv(ctx, ctx->compute, 't', rows, n, rb.vals[g], rb.idx32[g], rb.offs[g], xd + r0, yd, bnnz));
     }
     BOF_CUDA(ctx, cudaEventRecord(ev_done, ctx->compute));
     used[g] = true;
@@ -396,40 +433,19 @@ int bof_host_csrcsc(bof_ctx* ctx, int64_t m, int64_t n, const int64_t* ia, const
   BOF_CUDA(ctx, cudaSetDevice(ctx->device));
   stats_begin(ctx);
   CallGuard call_guard(ctx);
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice, D2H = cudaMemcpyDeviceToHost;
   const int64_t nnz = ia[m] - ia[0];
   BOF_REQUIRE(ctx, nnz >= 0 && nnz < (1ll << 31), "csrcsc: nnz must be in [0, 2^31)");
-  const size_t z = (size_t)std::max<int64_t>(nnz, 1);
-  int64_t *offs_d, *offs_t, *idx64;
-  int32_t *idx32, *idx_t;
-  float *vals_d, *vals_t;
-  void* ws;
-  const size_t wsb = csr2csc_workspace_bytes(m, n, nnz);
-  BOF_TRY(slot_reserve(ctx, S_OFFS, (size_t)m + 1, &offs_d));
-  BOF_TRY(slot_reserve(ctx, S_IDX64, z, &idx64));
-  BOF_TRY(slot_reserve(ctx, S_IDX32, z, &idx32));
-  BOF_TRY(slot_reserve(ctx, S_VALS, z, &vals_d));
-  BOF_TRY(slot_reserve(ctx, S_OUT0, (size_t)n + 1, &offs_t));
-  BOF_TRY(slot_reserve(ctx, S_OUT1, z, &idx_t));
-  BOF_TRY(slot_reserve(ctx, S_OUT2, z, &vals_t));
-  BOF_TRY(slot_reserve(ctx, S_WS, wsb, &ws));
-  // values ride a second stream so that both copy engines' queues stay busy
-  BOF_TRY(copy1d(ctx, offs_d, ia, (size_t)(m + 1) * 8, H2D, ctx->h2d));
-  BOF_TRY(copy1d(ctx, idx64, ja, (size_t)nnz * 8, H2D, ctx->h2d));
-  BOF_TRY(copy1d(ctx, vals_d, a, (size_t)nnz * 4, H2D, ctx->h2d));
-  cudaEvent_t ev = get_event(ctx, 0);
-  BOF_CUDA(ctx, cudaEventRecord(ev, ctx->h2d));
-  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev, 0));
-  BOF_TRY(launch_idx_narrow(ctx, ctx->compute, idx64, idx32, nnz));
-  BOF_TRY(launch_csr2csc(ctx, ctx->compute, m, n, nnz, offs_d, idx32, vals_d, offs_t, idx_t, vals_t, ws, wsb));
+  DevCsr at;
+  BOF_TRY(upload_transposed(ctx, m, n, nnz, a, ia, ja, EV_CSC_A, &at));
   // the int64 staging buffer of the input indices is free again: reuse it for the widened output
-  BOF_TRY(launch_idx_widen(ctx, ctx->compute, idx_t, idx64, nnz));
-  cudaEvent_t evk = get_event(ctx, 1);
-  BOF_CUDA(ctx, cudaEventRecord(evk, ctx->compute));
-  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h, evk, 0));
-  BOF_TRY(copy1d(ctx, a_tr, vals_t, (size_t)nnz * 4, D2H, ctx->d2h));
+  int64_t* idx64 = static_cast<int64_t*>(ctx->slot_ptr[S_IDX64]);
+  BOF_TRY(launch_idx_widen(ctx, ctx->compute, at.idx, idx64, nnz));
+  BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_CSC_T), ctx->compute));
+  BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h, get_event(ctx, EV_CSC_T), 0));
+  // values ride a second stream so that both copy engines' queues stay busy
+  BOF_TRY(copy1d(ctx, a_tr, at.vals, (size_t)nnz * 4, D2H, ctx->d2h));
   BOF_TRY(copy1d(ctx, ja_tr, idx64, (size_t)nnz * 8, D2H, ctx->compute));
-  BOF_TRY(copy1d(ctx, ia_tr, offs_t, (size_t)(n + 1) * 8, D2H, ctx->compute));  // offsets last, as csrcsc.cpp:150
+  BOF_TRY(copy1d(ctx, ia_tr, at.offs, (size_t)(n + 1) * 8, D2H, ctx->compute));  // offsets last, as csrcsc.cpp:150
   BOF_TRY(sync_all(ctx));
   stats_end(ctx);
   return call_guard.done();
@@ -484,38 +500,36 @@ int bof_csr_open(bof_ctx* ctx, int64_t m, int64_t n, const float* a, const int64
   const int64_t nnz = ia[m] - ia[0];
   BOF_REQUIRE(ctx, nnz >= 0 && nnz < (1ll << 31), "csr_open: nnz must be in [0, 2^31)");
   BOF_CUDA(ctx, cudaSetDevice(ctx->device));
+  // declared before the guard, so that a failed call quiesces the streams before the handle's memory is freed
+  std::unique_ptr<bof_csr, void (*)(bof_csr*)> h(new bof_csr(), csr_free);
   stats_begin(ctx);
   CallGuard call_guard(ctx);
-  bof_csr* h = new bof_csr();
   h->ctx = ctx; h->m = m; h->n = n; h->nnz = nnz;
-  auto guard = [&](int rc) { if (rc != BOF_OK) { quiesce(ctx); csr_free(h); } return rc; };
-  if (int rc = guard(csr_alloc(ctx, h, 0, m))) return rc;
+  BOF_TRY(csr_alloc(ctx, h.get(), 0, m));
   h->offs_host[0].assign(ia, ia + m + 1);
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice;
-  if (int rc = guard(copy1d(ctx, h->offs[0], ia, (size_t)(m + 1) * 8, H2D, ctx->h2d))) return rc;
-  if (int rc = guard(copy1d(ctx, h->vals[0], a, (size_t)nnz * 4, H2D, ctx->h2d))) return rc;
+  BOF_TRY(copy1d(ctx, h->offs[0], ia, (size_t)(m + 1) * 8, H2D, ctx->h2d));
+  BOF_TRY(copy1d(ctx, h->vals[0], a, (size_t)nnz * 4, H2D, ctx->h2d));
   // int64 column indices cross PCIe as they are on disk and are narrowed chunk by chunk (two staging generations)
   const int64_t chunk = std::max<int64_t>(std::min<int64_t>((int64_t)ctx->cfg.csrmm_max_nnz, nnz), 1);
   int64_t* st[2];
-  for (int g = 0; g < 2; ++g)
-    if (int rc = guard(slot_reserve(ctx, S_IDX64 + g, (size_t)chunk, &st[g]))) return rc;
+  for (int g = 0; g < 2; ++g) BOF_TRY(slot_reserve(ctx, S_IDX64 + g, (size_t)chunk, &st[g]));
   bool used[2] = {false, false};
   int ci = 0;
   for (int64_t z = 0; z < nnz; z += chunk, ++ci) {
     const int g = ci & 1;
     const int64_t cnt = std::min(chunk, nnz - z);
-    cudaEvent_t ev_up = get_event(ctx, 4 + g), ev_done = get_event(ctx, 6 + g);
-    if (used[g] && cudaStreamWaitEvent(ctx->h2d, ev_done, 0) != cudaSuccess) return guard(fail(ctx, BOF_ECUDA, "csr_open: wait failed"));
-    if (int rc = guard(copy1d(ctx, st[g], ja + z, (size_t)cnt * 8, H2D, ctx->h2d))) return rc;
-    cudaEventRecord(ev_up, ctx->h2d);
-    cudaStreamWaitEvent(ctx->compute, ev_up, 0);
-    if (int rc = guard(launch_idx_narrow(ctx, ctx->compute, st[g], h->idx[0] + z, cnt))) return rc;
-    cudaEventRecord(ev_done, ctx->compute);
+    cudaEvent_t ev_up = get_event(ctx, EV_UP + g), ev_done = get_event(ctx, EV_DONE + g);
+    if (used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, ev_done, 0));
+    BOF_TRY(copy1d(ctx, st[g], ja + z, (size_t)cnt * 8, H2D, ctx->h2d));
+    BOF_CUDA(ctx, cudaEventRecord(ev_up, ctx->h2d));
+    BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, ev_up, 0));
+    BOF_TRY(launch_idx_narrow(ctx, ctx->compute, st[g], h->idx[0] + z, cnt));
+    BOF_CUDA(ctx, cudaEventRecord(ev_done, ctx->compute));
     used[g] = true;
   }
-  if (int rc = guard(sync_all(ctx))) return rc;
+  BOF_TRY(sync_all(ctx));
   stats_end(ctx);
-  *out = h;
+  *out = h.release();
   return call_guard.done();
 }
 
@@ -526,13 +540,9 @@ int bof_csr_build_transpose(bof_csr* h) {
   BOF_CUDA(ctx, cudaSetDevice(ctx->device));
   CallGuard call_guard(ctx);
   BOF_TRY(csr_alloc(ctx, h, 1, h->n));
-  void* ws;
-  const size_t wsb = csr2csc_workspace_bytes(h->m, h->n, h->nnz);
-  BOF_TRY(slot_reserve(ctx, S_WS, wsb, &ws));
-  BOF_TRY(launch_csr2csc(ctx, ctx->compute, h->m, h->n, h->nnz, h->offs[0], h->idx[0], h->vals[0], h->offs[1],
-                         h->idx[1], h->vals[1], ws, wsb));
+  BOF_TRY(transpose_csr(ctx, h->m, h->n, h->nnz, h->offs[0], h->idx[0], h->vals[0], h->offs[1], h->idx[1], h->vals[1]));
   h->offs_host[1].resize((size_t)h->n + 1);
-  BOF_TRY(copy1d(ctx, h->offs_host[1].data(), h->offs[1], (size_t)(h->n + 1) * 8, cudaMemcpyDeviceToHost, ctx->compute));
+  BOF_TRY(copy1d(ctx, h->offs_host[1].data(), h->offs[1], (size_t)(h->n + 1) * 8, D2H, ctx->compute));
   BOF_TRY(sync_all(ctx));
   h->have_t = true;
   return call_guard.done();
@@ -568,10 +578,7 @@ int bof_csr_mm(bof_csr* h, char trans_a, int64_t k, float alpha, float beta, cha
   const int64_t out_rows = t ? h->n : h->m, in_rows = t ? h->m : h->n;
   if (out_rows == 0 || k == 0) { stats_end(ctx); return call_guard.done(); }
   const bool colmaj = ord_b == 'C';
-  const cudaMemcpyKind H2D = cudaMemcpyHostToDevice;
-  const float* vals = h->vals[t];
-  const int32_t* idx = h->idx[t];
-  const int64_t* offs = h->offs[t];
+  const HostC hc{c, colmaj ? out_rows : k, colmaj};
   const int64_t* oh = h->offs_host[t].data();
 
   // panel width: measured on the cfg-3 matrix at k = 256 (profiles/r01/resident_panel_sweep.txt): 32 -> 304 ms
@@ -589,25 +596,22 @@ int bof_csr_mm(bof_csr* h, char trans_a, int64_t k, float alpha, float beta, cha
     BOF_TRY(slot_reserve(ctx, S_CBLK + g, (size_t)std::min(rows_blk, out_rows) * kb, &cblk[g]));
     if (colmaj) BOF_TRY(slot_reserve(ctx, S_CBLK_T + g, (size_t)std::min(rows_blk, out_rows) * kb, &cblk_t[g]));
   }
-  // events: 0+gp panel uploaded, 2+gp panel consumed, 4+g old C block uploaded, 6+g block computed, 8+g block downloaded
   bool pan_used[2] = {false, false}, blk_used[2] = {false, false};
-  uint64_t down_ticket[2] = {0, 0};  // pageable C: the drainer enqueues the download and records event 8+g
+  uint64_t down_ticket[2] = {0, 0};  // pageable C: the drainer enqueues the download and records EV_DOWN + g
   auto upload_panel = [&](int p) -> int {
     const int gp = p & 1;
     const int64_t j0 = (int64_t)p * kb, kbp = std::min(kb, k - j0);
     float* bp = bpan_all + (size_t)gp * pan_elems;
-    if (pan_used[gp]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, 2 + gp), 0));
+    if (pan_used[gp]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, EV_PAN_FREE + gp), 0));
     if (in_rows > 0) {
       if (colmaj) {
         float* raw = braw_all + (size_t)gp * pan_elems;  // columns j0.. of a column-major B are contiguous
         BOF_TRY(copy1d(ctx, raw, b + j0 * in_rows, (size_t)in_rows * kbp * 4, H2D, ctx->h2d));
-      } else if (npan == 1) {
-        BOF_TRY(copy1d(ctx, bp, b, (size_t)in_rows * k * 4, H2D, ctx->h2d));
       } else {
         BOF_TRY(copy2d(ctx, bp, (size_t)kbp * 4, b + j0, (size_t)k * 4, (size_t)kbp * 4, (size_t)in_rows, H2D, ctx->h2d));
       }
     }
-    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, 0 + gp), ctx->h2d));
+    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_PAN + gp), ctx->h2d));
     pan_used[gp] = true;
     return BOF_OK;
   };
@@ -618,45 +622,34 @@ int bof_csr_mm(bof_csr* h, char trans_a, int64_t k, float alpha, float beta, cha
     const int64_t r0 = (int64_t)i * rows_blk, rows = std::min(rows_blk, out_rows - r0);
     const int64_t z0 = oh[r0] - oh[0];
     float* bp = bpan_all + (size_t)gp * pan_elems;
-    float* c_io = colmaj ? cblk_t[g] : cblk[g];
-    if (blk_used[g]) d2h_fence(ctx, down_ticket[g]);  // event 8+g recorded, 6+g may be re-recorded
+    if (blk_used[g]) d2h_fence(ctx, down_ticket[g]);  // EV_DOWN + g recorded, EV_DONE + g may be re-recorded
     if (beta != 0.f) {
       if (blk_used[g]) {
-        BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, 6 + g), 0));
-        BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, 8 + g), 0));
+        BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, EV_DONE + g), 0));
+        BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->h2d, get_event(ctx, EV_DOWN + g), 0));
       }
-      if (colmaj) BOF_TRY(copy2d(ctx, c_io, (size_t)rows * 4, c + j0 * out_rows + r0, (size_t)out_rows * 4, (size_t)rows * 4, (size_t)kbp, H2D, ctx->h2d));
-      else BOF_TRY(copy2d(ctx, c_io, (size_t)kbp * 4, c + r0 * k + j0, (size_t)k * 4, (size_t)kbp * 4, (size_t)rows, H2D, ctx->h2d));
-      BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, 4 + g), ctx->h2d));
-      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, 4 + g), 0));
+      BOF_TRY(upload_c_block(ctx, hc, r0, rows, j0, kbp, colmaj ? cblk_t[g] : cblk[g]));
+      BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_UP + g), ctx->h2d));
+      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_UP + g), 0));
     }
     if (i == 0) {
-      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, 0 + gp), 0));
+      BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_PAN + gp), 0));
       if (colmaj && in_rows > 0)
         BOF_TRY(launch_transpose(ctx, ctx->compute, kbp, in_rows, braw_all + (size_t)gp * pan_elems, in_rows, bp, kbp));
     }
-    if (blk_used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, 8 + g), 0));
-    if (colmaj) {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, rows, kbp, 1.f, vals + z0, idx + z0, offs + r0, bp, kbp, 0.f, cblk[g], kbp));
-      BOF_TRY(launch_transpose_axpby(ctx, ctx->compute, rows, kbp, alpha, cblk[g], kbp, beta, cblk_t[g], rows));
-    } else {
-      BOF_TRY(launch_spmm_rm(ctx, ctx->compute, rows, kbp, alpha, vals + z0, idx + z0, offs + r0, bp, kbp, beta, cblk[g], kbp));
-    }
-    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, 6 + g), ctx->compute));
-    if (i == nblk - 1) BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, 2 + gp), ctx->compute));
+    if (blk_used[g]) BOF_CUDA(ctx, cudaStreamWaitEvent(ctx->compute, get_event(ctx, EV_DOWN + g), 0));
+    const DevCsr blk{h->offs[t] + r0, h->idx[t] + z0, h->vals[t] + z0};
+    BOF_TRY(spmm_c_block(ctx, rows, kbp, alpha, blk, bp, 0, beta, cblk[g], cblk_t[g]));
+    BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_DONE + g), ctx->compute));
+    if (i == nblk - 1) BOF_CUDA(ctx, cudaEventRecord(get_event(ctx, EV_PAN_FREE + gp), ctx->compute));
     blk_used[g] = true;
     return BOF_OK;
   };
   auto fetch_block = [&](int p, int i, int g) -> int {
     const int64_t j0 = (int64_t)p * kb, kbp = std::min(kb, k - j0);
     const int64_t r0 = (int64_t)i * rows_blk, rows = std::min(rows_blk, out_rows - r0);
-    float* c_io = colmaj ? cblk_t[g] : cblk[g];
-    cudaEvent_t ev_done = get_event(ctx, 6 + g), ev_down = get_event(ctx, 8 + g);
-    uint64_t* tk = &down_ticket[g];
-    if (colmaj) BOF_TRY(d2h_transfer(ctx, c + j0 * out_rows + r0, (size_t)out_rows * 4, c_io, (size_t)rows * 4, (size_t)rows * 4, (size_t)kbp, ctx->d2h, ev_done, ev_down, tk));
-    else if (npan == 1) BOF_TRY(d2h_transfer(ctx, c + r0 * k, (size_t)rows * k * 4, c_io, (size_t)rows * k * 4, (size_t)rows * k * 4, 1, ctx->d2h, ev_done, ev_down, tk));
-    else BOF_TRY(d2h_transfer(ctx, c + r0 * k + j0, (size_t)k * 4, c_io, (size_t)kbp * 4, (size_t)kbp * 4, (size_t)rows, ctx->d2h, ev_done, ev_down, tk));
-    return BOF_OK;
+    return download_c_block(ctx, hc, r0, rows, j0, kbp, colmaj ? cblk_t[g] : cblk[g], get_event(ctx, EV_DONE + g),
+                            get_event(ctx, EV_DOWN + g), &down_ticket[g]);
   };
   // software pipeline over (panel, block): launch step s, then download step s-1
   BOF_TRY(upload_panel(0));
@@ -694,11 +687,11 @@ int bof_csr_mv(bof_csr* h, char trans_a, const float* x, float* y) {
   BOF_TRY(slot_reserve(ctx, S_MISC, (size_t)std::max<int64_t>(xlen, 1), &xd));
   BOF_TRY(slot_reserve(ctx, S_OUT0, (size_t)ylen, &yd));
   cudaStream_t s = ctx->compute;
-  BOF_TRY(copy1d(ctx, xd, x, (size_t)xlen * 4, cudaMemcpyHostToDevice, s));
+  BOF_TRY(copy1d(ctx, xd, x, (size_t)xlen * 4, H2D, s));
   if (!tr) BOF_TRY(launch_spmv(ctx, s, 'N', h->m, h->n, h->vals[0], h->idx[0], h->offs[0], xd, yd));
   else if (h->have_t) BOF_TRY(launch_spmv(ctx, s, 'N', h->n, h->m, h->vals[1], h->idx[1], h->offs[1], xd, yd));
   else BOF_TRY(launch_spmv(ctx, s, 'T', h->m, h->n, h->vals[0], h->idx[0], h->offs[0], xd, yd, h->nnz));
-  BOF_TRY(copy1d(ctx, y, yd, (size_t)ylen * 4, cudaMemcpyDeviceToHost, s));
+  BOF_TRY(copy1d(ctx, y, yd, (size_t)ylen * 4, D2H, s));
   BOF_TRY(sync_all(ctx));
   stats_end(ctx);
   return call_guard.done();
