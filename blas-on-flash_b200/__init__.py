@@ -1,4 +1,4 @@
-"""bof_b200 -- B200-native hot path of BLAS-on-Flash (csrmm, gemm, csrgemv, csrcsc, kmeans step).
+"""bof_b200 -- B200-native hot path of BLAS-on-Flash (csrmm, gemm, gemv, csrgemv, csrcsc, kmeans step).
 
 The product is ``libbof_b200.so`` (hand-written sm_100a kernels + C ABI, ``include/bof_b200.h``)
 and the C++ adapters that keep the reference's ``flash::`` signatures (``include/flash_blas.h``).
@@ -99,6 +99,16 @@ class Context:
         self._check(self.lib.bof_sgemm_f32(self.h, stream or _cur_stream(), ch(ord_), ch(ta), ch(tb), m, n, k, alpha,
                                            ptr(A), lda, ptr(B), ldb, beta, ptr(Cmat), ldc, ptr(ws), ws.numel()))
 
+    def sgemv_workspace(self, ord_, trans, m, n):
+        return self._ws(self.lib.bof_sgemv_workspace_bytes(ch(ord_), ch(trans), m, n))
+
+    def sgemv(self, ord_, trans, m, n, alpha, A, lda, x, beta, y, ws=None, stream=None):
+        """y = alpha * op(A) x + beta * y on device tensors (A stored 'R' / 'C' with leading dimension lda, 0 = tight)"""
+        if ws is None:
+            ws = self.sgemv_workspace(ord_, trans, m, n)
+        self._check(self.lib.bof_sgemv_f32(self.h, stream or _cur_stream(), ch(ord_), ch(trans), m, n, alpha, ptr(A), lda,
+                                           ptr(x), beta, ptr(y), ptr(ws), ws.numel()))
+
     def tc_issue_rate(self, kind: int, rounds: int = 20000, stream=None):
         """(mma_tflops, useful_tflops) of the tensor-pipe issue-rate microbenchmark; kind 0 tf32, 1 bf16, 2 hybrid mix"""
         a, b = C.c_double(), C.c_double()
@@ -157,6 +167,9 @@ class Context:
     def host_csrmm_devb(self, m, n, k, alpha, beta, a, ia, ja, b_dev, c):
         self._check(self.lib.bof_host_csrmm_devb(self.h, m, n, k, alpha, beta, ptr(a), ptr(ia), ptr(ja), ptr(b_dev),
                                                  ptr(c)))
+
+    def host_gemv(self, ord_, trans, m, n, alpha, beta, a, x, y, lda=0):
+        self._check(self.lib.bof_host_gemv(self.h, ch(ord_), ch(trans), m, n, alpha, beta, ptr(a), lda, ptr(x), ptr(y)))
 
     def host_csrgemv(self, trans_a, m, n, a, ia, ja, b, c):
         self._check(self.lib.bof_host_csrgemv(self.h, ch(trans_a), m, n, ptr(a), ptr(ia), ptr(ja), ptr(b), ptr(c)))
@@ -301,6 +314,9 @@ class MultiGpu:
 
     def csrgemv(self, trans_a, m, n, a, ia, ja, x, y):
         self._check(self.lib.bof_mgpu_csrgemv(self.h, ch(trans_a), m, n, ptr(a), ptr(ia), ptr(ja), ptr(x), ptr(y)))
+
+    def gemv(self, ord_, trans, m, n, alpha, beta, a, x, y, lda=0):
+        self._check(self.lib.bof_mgpu_gemv(self.h, ch(ord_), ch(trans), m, n, alpha, beta, ptr(a), lda, ptr(x), ptr(y)))
 
     def kmeans_lloyd(self, npoints, ncenters, dim, points, centers, iters, assign=None):
         self._check(self.lib.bof_mgpu_kmeans_lloyd(self.h, npoints, ncenters, dim, ptr(points), ptr(centers), iters,

@@ -68,6 +68,8 @@ PROTOTYPES = {
     "bof_sgemm_f32": (C.c_int, [_vp, _vp, _ch, _ch, _ch, _i64, _i64, _i64, _f32, _vp, _i64, _vp, _i64, _f32,
                                 _vp, _i64, _vp, _sz]),
     "bof_sgemm_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "bof_sgemv_f32": (C.c_int, [_vp, _vp, _ch, _ch, _i64, _i64, _f32, _vp, _i64, _vp, _f32, _vp, _vp, _sz]),
+    "bof_sgemv_workspace_bytes": (_sz, [_ch, _ch, _i64, _i64]),
     "bof_tc_issue_rate": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "bof_csr2csc": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz]),
     "bof_csr2csc_workspace_bytes": (_sz, [_i64, _i64, _i64]),
@@ -86,6 +88,7 @@ PROTOTYPES = {
     "bof_host_csrmm_devb": (C.c_int, [_vp, _i64, _i64, _i64, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
     "bof_host_kmeans_dist": (C.c_int, [_vp, _ch, _ch, _ch, _i64, _i64, _i64, _f32, _f32, _vp, _vp, _vp, _i64, _i64, _i64,
                                        _vp, _vp]),
+    "bof_host_gemv": (C.c_int, [_vp, _ch, _ch, _i64, _i64, _f32, _f32, _vp, _i64, _vp, _vp]),
     "bof_host_csrgemv": (C.c_int, [_vp, _ch, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "bof_host_csrcsc": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bof_csr_open": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, C.POINTER(_vp)]),
@@ -116,6 +119,7 @@ PROTOTYPES = {
     "bof_mgpu_gemm": (C.c_int, [_vp, _ch, _ch, _ch, _i64, _i64, _i64, _f32, _f32, _vp, _vp, _vp, _i64, _i64, _i64]),
     "bof_mgpu_csrmm": (C.c_int, [_vp, _ch, _i64, _i64, _i64, _f32, _f32, _vp, _vp, _vp, _ch, _vp, _vp]),
     "bof_mgpu_csrgemv": (C.c_int, [_vp, _ch, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "bof_mgpu_gemv": (C.c_int, [_vp, _ch, _ch, _i64, _i64, _f32, _f32, _vp, _i64, _vp, _vp]),
     "bof_mgpu_kmeans_lloyd": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _i64, _vp]),
     "bof_kmeans_close": (C.c_int, [_vp]),
 }

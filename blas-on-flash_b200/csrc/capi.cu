@@ -167,6 +167,23 @@ int bof_sgemm_f32(bof_ctx* ctx, void* stream, char ord, char ta, char tb, int64_
   return gemm_canon_device(ctx, as_stream(stream), c, alpha, beta, C, workspace, workspace_bytes);
 }
 
+size_t bof_sgemv_workspace_bytes(char ord, char trans, int64_t m, int64_t n) {
+  GemvCanon c;
+  if (canon_gemv(nullptr, ord, trans, m, n, 0, &c) != BOF_OK) return 0;
+  return gemv_workspace_bytes(c);
+}
+
+int bof_sgemv_f32(bof_ctx* ctx, void* stream, char ord, char trans, int64_t m, int64_t n, float alpha, const float* A,
+                  int64_t lda, const float* x, float beta, float* y, void* workspace, size_t workspace_bytes) {
+  if (!ctx) return BOF_EINVAL;
+  GemvCanon c;
+  BOF_TRY(canon_gemv(ctx, ord, trans, m, n, lda, &c));
+  const size_t need = gemv_workspace_bytes(c);
+  BOF_REQUIRE(ctx, need == 0 || (workspace && workspace_bytes >= need),
+              "gemv: needs bof_sgemv_workspace_bytes() = %zu bytes of workspace", need);
+  return launch_gemv(ctx, as_stream(stream), c, A, x, nullptr, nullptr, alpha, beta, y, true, workspace);
+}
+
 int bof_tc_issue_rate(bof_ctx* ctx, void* stream, int kind, int rounds, double* mma_tflops, double* useful_tflops) {
   if (!ctx) return BOF_EINVAL;
   BOF_CUDA(ctx, cudaSetDevice(ctx->device));

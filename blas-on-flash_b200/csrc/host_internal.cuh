@@ -83,6 +83,24 @@ int64_t k_chunk_of(const bof_ctx* ctx);
 int gemm_canon_device(bof_ctx* ctx, cudaStream_t s, const Canon& c, float alpha, float beta, float* C,
                       void* ws, size_t ws_bytes);
 
+// ---- gemv.cu / gemv_host.cu ----
+// Canonical form of a gemv: the stored matrix S (rows x cols, row-major, pitch ld) and either one dot product per row
+// of S (row-dot: ('R','N'), ('C','T')) or one sum per column (column-sum: ('R','T'), ('C','N')).
+struct GemvCanon {
+  int64_t rows, cols, ld;
+  bool rowdot;
+  int64_t nout() const { return rowdot ? rows : cols; }   // length of y
+  int64_t nred() const { return rowdot ? cols : rows; }   // length of x
+};
+int canon_gemv(bof_ctx* ctx, char ord, char trans, int64_t m, int64_t n, int64_t lda, GemvCanon* out);
+int64_t gemv_chunks(int64_t len);   // BOF_GEMV_CHUNK pieces of a reduction of length len
+size_t gemv_workspace_bytes(const GemvCanon& c);
+// y[o] (o < nout) of the canonical problem on device S, x, y.  carry (may be null) seeds the fold of every output with a
+// partial sum of earlier reduction chunks (S and x then start on a chunk boundary of the whole reduction);
+// final_out: y = alpha*acc + beta*y, else acc_out = acc (carry and acc_out may alias).  ws: gemv_workspace_bytes(c).
+int launch_gemv(bof_ctx* ctx, cudaStream_t s, const GemvCanon& c, const float* S, const float* x, const float* carry,
+                float* acc_out, float alpha, float beta, float* y, bool final_out, void* ws);
+
 // ---- comm.cu: communicator rank of a context (world 1 / rank 0 without one) ----
 int comm_world(const bof_ctx* ctx);
 int comm_rank(const bof_ctx* ctx);

@@ -243,6 +243,33 @@ int bof_mgpu_csrgemv(bof_mgpu* mg, char trans_a, int64_t m, int64_t n, const flo
   return BOF_OK;
 }
 
+// flash::gemv over the GPUs: the outputs are split, never the reduction.  Row-dot shapes give each GPU a range of rows
+// of the stored matrix, column sums a range of its columns (same lda, offset base); every GPU uploads its own x.
+int bof_mgpu_gemv(bof_mgpu* mg, char ord, char trans, int64_t m, int64_t n, float alpha, float beta, const float* a,
+                  int64_t lda, const float* x, float* y) {
+  if (!mg || mg->ctx.empty()) return BOF_EINVAL;
+  const int world = (int)mg->ctx.size();
+  GemvCanon c;
+  if (int rc = canon_gemv(mg->ctx[0], ord, trans, m, n, lda, &c)) {
+    mg->err = bof_last_error(mg->ctx[0]);
+    return rc;
+  }
+  if (world == 1 || c.nout() < world) {
+    const int rc = bof_host_gemv(mg->ctx[0], ord, trans, m, n, alpha, beta, a, lda, x, y);
+    if (rc != BOF_OK) mg->err = bof_last_error(mg->ctx[0]);
+    return rc;
+  }
+  return for_each_rank(mg, [&](int r) {
+    int64_t o0, o1;
+    split_rows(c.nout(), world, r, 1, &o0, &o1);
+    if (o1 == o0) return (int)BOF_OK;
+    // the part as a row-major problem on the stored matrix: ('R','N') is a row-dot, ('R','T') a column sum
+    if (c.rowdot)
+      return bof_host_gemv(mg->ctx[r], 'R', 'N', o1 - o0, c.cols, alpha, beta, a + o0 * c.ld, c.ld, x, y + o0);
+    return bof_host_gemv(mg->ctx[r], 'R', 'T', c.rows, o1 - o0, alpha, beta, a + o0, c.ld, x, y + o0);
+  });
+}
+
 // `iters` Lloyd iterations (drivers/in_mem_kmeans.cpp:89-152), points sharded over the GPUs and resident, one NCCL
 // allreduce of [sums | counts] per iteration.  centers_host: initial centres in, final centres out; assign_out
 // (npoints entries, may be NULL): assignment of the last iteration.

@@ -20,7 +20,7 @@ std::mutex g_mu;
 bof_ctx* g_ctx = nullptr;
 bof_mgpu* g_mgpu = nullptr;   // BOF_GPUS > 1: one context per GPU in this process, g_ctx = its rank 0
 
-// BOF_GPUS=<n> | all : spread gemm / csrmm / csrgemv / kmeans_lloyd over the GPUs of the node (default: one GPU)
+// BOF_GPUS=<n> | all : spread gemm / gemv / csrmm / csrgemv / kmeans_lloyd over the GPUs of the node (default: one GPU)
 int env_gpus() {
   const char* v = std::getenv("BOF_GPUS");
   if (!v) return 1;
@@ -104,6 +104,21 @@ FBLAS_INT gemm(CHAR mat_ord, CHAR trans_a, CHAR trans_b, FBLAS_UINT m, FBLAS_UIN
                                       b.ptr, c.ptr, (int64_t)lda_a, (int64_t)lda_b, (int64_t)lda_c));
   return done("gemm", bof_host_gemm(ctx, mat_ord, trans_a, trans_b, (int64_t)m, (int64_t)n, (int64_t)k, alpha, beta,
                                     a.ptr, b.ptr, c.ptr, (int64_t)lda_a, (int64_t)lda_b, (int64_t)lda_c));
+}
+
+FBLAS_INT gemv(CHAR mat_ord, CHAR trans_a, FBLAS_UINT m, FBLAS_UINT n, FPTYPE alpha, FPTYPE beta, flash_ptr<FPTYPE> a,
+               flash_ptr<FPTYPE> b, flash_ptr<FPTYPE> c, FBLAS_UINT lda_a) {
+  return gemv(mat_ord, trans_a, m, n, alpha, beta, a, b.ptr, c.ptr, lda_a);
+}
+
+FBLAS_INT gemv(CHAR mat_ord, CHAR trans_a, FBLAS_UINT m, FBLAS_UINT n, FPTYPE alpha, FPTYPE beta, flash_ptr<FPTYPE> a,
+               FPTYPE* b, FPTYPE* c, FBLAS_UINT lda_a) {
+  bof_ctx* ctx = flash_context();
+  if (!ctx) return -1;
+  if (multi())
+    return done("gemv", bof_mgpu_gemv(g_mgpu, mat_ord, trans_a, (int64_t)m, (int64_t)n, alpha, beta, a.ptr, (int64_t)lda_a,
+                                      b, c));
+  return done("gemv", bof_host_gemv(ctx, mat_ord, trans_a, (int64_t)m, (int64_t)n, alpha, beta, a.ptr, (int64_t)lda_a, b, c));
 }
 
 FBLAS_INT kmeans(CHAR mat_ord, CHAR trans_a, CHAR trans_b, FBLAS_UINT m, FBLAS_UINT n, FBLAS_UINT k, FPTYPE alpha,

@@ -172,6 +172,23 @@ BOF_API int bof_csr2csc(bof_ctx* ctx, void* stream, int64_t m, int64_t n, int64_
                 int32_t* idx_t, float* vals_t, void* workspace, size_t workspace_bytes);
 BOF_API size_t bof_csr2csc_workspace_bytes(int64_t m, int64_t n, int64_t nnz);
 
+/* K12: y = alpha * op(A) * x + beta * y, fp32 (cblas_sgemv with incx = incy = 1; flash::gemv, which the reference
+ * declares in include/flash_blas.h:28-30 but never defines).  A is m x n, stored ord 'R' (row-major) or 'C'
+ * (column-major) with leading dimension lda (0 = tight: n for 'R', m for 'C').  trans 'N': x has n entries, y has m;
+ * 'T': x has m entries, y has n.  beta == 0 => y is not read.  alpha == 0 is not a shortcut: an Inf or NaN in A or x
+ * reaches exactly the outputs whose dot product it enters.  An empty reduction (n == 0 for 'N', m == 0 for 'T') gives
+ * y = beta * y (0 when beta == 0).
+ * Deterministic: the reduction is cut into chunks of BOF_GEMV_CHUNK elements, each summed by a fixed tree over the
+ * element positions, and the chunk sums are added in ascending order into one fp32 accumulator before alpha and beta
+ * are applied.  bof_sgemv_f32, bof_host_gemv and bof_mgpu_gemv therefore give the same bits for the same problem,
+ * whatever the tiling, the alignment, lda or the number of GPUs; so do ('R','N') and ('C','T') on the same memory.
+ * Needs bof_sgemv_workspace_bytes() of workspace (0 for an empty problem). */
+#define BOF_GEMV_CHUNK 4096
+BOF_API int bof_sgemv_f32(bof_ctx* ctx, void* stream, char ord, char trans, int64_t m, int64_t n, float alpha,
+                  const float* A, int64_t lda, const float* x, float beta, float* y, void* workspace,
+                  size_t workspace_bytes);
+BOF_API size_t bof_sgemv_workspace_bytes(char ord, char trans, int64_t m, int64_t n);
+
 /* K11: out[r] = sum_j X[r, j]^2 for a row-major rows x dim matrix.
  * Replaces the cblas_sdot loops of drivers/in_mem_kmeans.cpp:75-78,179-182. */
 BOF_API int bof_row_sqnorm_f32(bof_ctx* ctx, void* stream, int64_t rows, int64_t dim, const float* X,
@@ -288,6 +305,11 @@ BOF_API int bof_mgpu_csrmm(bof_mgpu* mg, char trans_a, int64_t m, int64_t n, int
 /* flash::csrgemv: 'N' disjoint row blocks; 'T' per-GPU partial y added on the host in GPU order (deterministic). */
 BOF_API int bof_mgpu_csrgemv(bof_mgpu* mg, char trans_a, int64_t m, int64_t n, const float* a, const int64_t* ia,
                      const int64_t* ja, const float* x, float* y);
+/* flash::gemv: the outputs are split over the GPUs (rows of the stored matrix for ('R','N') / ('C','T'), its columns
+ * otherwise); every GPU runs bof_host_gemv on its part with its own copy of x.  No collective, no host-side sum: the
+ * result is bit-identical to one GPU.  Fewer outputs than GPUs runs on GPU 0. */
+BOF_API int bof_mgpu_gemv(bof_mgpu* mg, char ord, char trans, int64_t m, int64_t n, float alpha, float beta,
+                  const float* a, int64_t lda, const float* x, float* y);
 /* drivers/in_mem_kmeans.cpp:89-152 x iters: points sharded and resident, NCCL allreduce per iteration. */
 BOF_API int bof_mgpu_kmeans_lloyd(bof_mgpu* mg, int64_t npoints, int64_t ncenters, int64_t dim,
                           const float* points_host, float* centers_host, int64_t iters, int64_t* assign_out);
@@ -300,6 +322,14 @@ BOF_API int bof_host_kmeans_dist(bof_ctx* ctx, char mat_ord, char trans_a, char 
                          int64_t k, float alpha, float beta, const float* a, const float* b, float* c,
                          int64_t lda_a, int64_t lda_b, int64_t lda_c, const float* c_l2sq,
                          const float* p_l2sq);
+
+/* flash::gemv with A, x and y in host memory (pageable, pinned or a map_file mapping); arguments as bof_sgemv_f32.
+ * A crosses PCIe exactly once, in tiles of at most BOF_GEMV_BLOCK_BYTES (environment, read on every call; default
+ * 128 MiB, smaller so that a large A makes at least 8 tiles), so A may exceed HBM.  Tiles along the reduction start on
+ * BOF_GEMV_CHUNK boundaries and the fp32 fold of every output stays on the device across them, which keeps the result
+ * bit-identical to bof_sgemv_f32.  bof_stats: h2d_bytes = sz(A) + sz(x) + (beta != 0) sz(y), d2h_bytes = sz(y). */
+BOF_API int bof_host_gemv(bof_ctx* ctx, char ord, char trans, int64_t m, int64_t n, float alpha, float beta,
+                  const float* a, int64_t lda, const float* x, float* y);
 
 /* flash::csrgemv (include/flash_blas.h:55-57; src/blas/csrgemv.cpp:82-97). */
 BOF_API int bof_host_csrgemv(bof_ctx* ctx, char trans_a, int64_t m, int64_t n, const float* a,

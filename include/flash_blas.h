@@ -5,8 +5,7 @@
 // runs in hand-written sm_100a kernels.  Return convention as the reference: 0 on success, -1 on a
 // bad argument (src/blas/csrmm.cpp:433-449) or any CUDA / I/O failure (message on stderr).
 //
-// Out of scope of the hot path (SURVEY.md section 2): flash::gemv (declared but never defined in the
-// reference), sort, map, reduce.
+// Out of scope of the hot path (SURVEY.md section 2): sort, map, reduce.
 #pragma once
 
 #include "bof_types.h"
@@ -23,6 +22,15 @@ FBLAS_INT gemm(CHAR mat_ord, CHAR trans_a, CHAR trans_b,
                FPTYPE alpha, FPTYPE beta,
                flash_ptr<FPTYPE> a, flash_ptr<FPTYPE> b, flash_ptr<FPTYPE> c,
                FBLAS_UINT lda_a = 0, FBLAS_UINT lda_b = 0, FBLAS_UINT lda_c = 0);
+
+// c = alpha * op(A) * b + beta * c                            [declared, never defined: reference flash_blas.h:28-30]
+//   A is m x n stored mat_ord 'R' | 'C' with leading dimension lda_a (0 = tight), trans_a 'N' | 'T';
+//   b has n ('N') or m ('T') entries, c the other count.  beta == 0: c is not read.  Deterministic, and the same bits
+//   on one GPU or several (bof_host_gemv / bof_mgpu_gemv).  The FPTYPE* overload takes b and c in host memory.
+FBLAS_INT gemv(CHAR mat_ord, CHAR trans_a, FBLAS_UINT m, FBLAS_UINT n, FPTYPE alpha, FPTYPE beta,
+               flash_ptr<FPTYPE> a, flash_ptr<FPTYPE> b, flash_ptr<FPTYPE> c, FBLAS_UINT lda_a = 0);
+FBLAS_INT gemv(CHAR mat_ord, CHAR trans_a, FBLAS_UINT m, FBLAS_UINT n, FPTYPE alpha, FPTYPE beta,
+               flash_ptr<FPTYPE> a, FPTYPE* b, FPTYPE* c, FBLAS_UINT lda_a = 0);
 
 // Distance tile of k-means: C = alpha * op(A) * op(B) + beta * C + c_l2sq 1^T + 1 p_l2sq^T
 //                                                                        [reference flash_blas.h:20-25]
